@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the BiSinger synthesis hot path on B200 (contract: see the task brief / DESIGN.md §7).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--precision bf16x3|bf16]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--precision bf16x3|bf16] [--dump-outputs DIR]
 
 Metric (BASELINE.json): seconds of audio synthesised per wall-second, diffusion mel (K=100 DiffNet sampler) + HiFi-GAN/NSF
 vocoder.  Workload at every N: cfg3 = one batch of 32 x 10 s phrases (T = 1875 mel frames, 24 kHz, hop 128) per rank per
@@ -106,6 +106,24 @@ class ClockSampler:
                 "samples": len(sm)}
 
 
+DUMP_BYTES = 60 << 20
+
+
+def dump_outputs(d, arrays):
+    """Writes each array as d/<name>.npy in float32.  When they hold more than DUMP_BYTES in all, each one is cut to a sample of its
+    elements (its share of the budget, flat indices drawn with a fixed seed and sorted), so that runs with the same arguments write
+    the same elements and two builds can be compared output for output."""
+    import numpy as np
+    os.makedirs(d, exist_ok=True)
+    total = sum(a.size * 4 for a in arrays.values())
+    for name, a in arrays.items():
+        a = np.ascontiguousarray(a, dtype=np.float32)
+        if total > DUMP_BYTES:
+            idx = np.random.default_rng(0).choice(a.size, a.size * DUMP_BYTES // total, replace=False)
+            a = a.reshape(-1)[np.sort(idx)]
+        np.save(os.path.join(d, name + ".npy"), a)
+
+
 def build_models(dev, precision):
     import torch
     from bisinger_b200 import synthetic as synth   # seeded random-init weights of the named architecture (no checkpoints reachable)
@@ -165,7 +183,7 @@ def run_ours(args):
 
     def step_resident(i):
         mel = gd.sample(cond_d, mel_d, seed=i)                          # [B,T,80]
-        return gen(mel.transpose(1, 2).contiguous(), f0_d, seed=i)      # [B,1,T*hop]
+        return mel, gen(mel.transpose(1, 2).contiguous(), f0_d, seed=i)  # [B,1,T*hop]
 
     def step_e2e(i):
         c = cond_p.to(dev, non_blocking=True); m = mel_p.to(dev, non_blocking=True); f = f0_p.to(dev, non_blocking=True)
@@ -187,8 +205,9 @@ def run_ours(args):
             cs.start()
         n0 = launch_count()
         e0.record(stream)
-        for i in range(steps):
+        for i in range(steps - 1):
             fn(i)
+        out = fn(steps - 1)                 # only the last step's result is held, as a caller of the path would hold it
         e1.record(stream)
         barrier()
         ms = e0.elapsed_time(e1)
@@ -198,14 +217,17 @@ def run_ours(args):
             t = torch.tensor([ms], dtype=torch.float64, device=dev)
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             ms = float(t.item())
-        return ms, n1 - n0, clocks
+        return ms, n1 - n0, clocks, out
 
     for i in range(args.warmup):
         step_resident(i)
-    ms, launches, clocks = timed(step_resident, args.steps, sample_clocks=True)
+    ms, launches, clocks, last = timed(step_resident, args.steps, sample_clocks=True)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"mel": last[0].cpu().numpy(), "wav": last[1].cpu().numpy()})
+    del last
     for i in range(max(1, args.warmup // 2)):
         step_e2e(i)
-    ms_e2e, _, _ = timed(step_e2e, args.steps)
+    ms_e2e, _, _, _ = timed(step_e2e, args.steps)
 
     value = world * args.steps * audio_s / (ms / 1e3)
     e2e = world * args.steps * audio_s / (ms_e2e / 1e3)
@@ -537,7 +559,8 @@ def run_reference(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=None,
+                    help="timed steps (default 5); cfg5 times its share of the --phrases batches instead and rejects --steps")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--precision", default="fp16x2", choices=["fp16x2", "bf16x3", "bf16"])
@@ -548,7 +571,17 @@ def main():
     ap.add_argument("--phrases", type=int, default=4096)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-eager-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the mel [B,T,80] and waveform [B,1,T*hop] of the last timed step (cfg3, rank 0) as DIR/mel.npy and "
+                         "DIR/wav.npy, float32; past 60 MiB in all a fixed seeded sample of each")
     args = ap.parse_args()
+    if args.workload == "cfg5" and args.steps is not None:
+        ap.error("--steps does not apply to --workload cfg5: it times every batch of --phrases")
+    args.steps = 5 if args.steps is None else args.steps
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "cfg3"):
+        ap.error("--dump-outputs needs --impl ours and --workload cfg3")
     if args.impl == "reference":
         run_reference(args)
         return

@@ -133,7 +133,7 @@ def test_from_reference_copies_a_live_encoder_block_stack():
     block weight taken over by name, no positional term (the encoder's stack is FFTBlocks(use_pos_embed=False))."""
     import ref_shim
     if not ref_shim.available():
-        pytest.skip("reference tree not present (GPU box)")
+        pytest.skip("needs the original BiSinger source tree (set BISINGER_REFERENCE)")
     from make_golden_fft import FFT_HP
     ns = ref_shim.load()
     ns.hparams.update(FFT_HP)
@@ -166,7 +166,7 @@ def test_device_blocks_encoder_is_the_reference_midi_encoder_with_the_block_stac
     that call with the oracle's FFT blocks and comparing with the reference encoder's own eval forward."""
     import ref_shim
     if not ref_shim.available():
-        pytest.skip("reference tree not present (GPU box)")
+        pytest.skip("needs the original BiSinger source tree (set BISINGER_REFERENCE)")
     from make_golden_fft import FFT_HP
     ns = ref_shim.load()
     ns.hparams.update({**FFT_HP, "rel_pos": True})

@@ -110,7 +110,7 @@ def test_fp16x2_model_meets_mel_tolerance(sd_diff):
 reference_present = __import__("ref_shim").available()
 
 
-@pytest.mark.skipif(not reference_present, reason="/root/reference not mounted (GPU box)")
+@pytest.mark.skipif(not reference_present, reason="needs the original BiSinger source tree (set BISINGER_REFERENCE)")
 def test_live_reference_matches_oracle(sd_diff):
     """Build container only: run the unmodified reference DiffNet on fresh inputs and compare with the restatement."""
     import ref_shim
@@ -173,7 +173,7 @@ def test_forward_golden_vs_oracle(sd_diff):
             assert float(np.abs(ref[-1, c["T"] - c["pad_tail"]:]).max()) == 0.0
 
 
-@pytest.mark.skipif(not reference_present, reason="/root/reference not mounted (GPU box)")
+@pytest.mark.skipif(not reference_present, reason="needs the original BiSinger source tree (set BISINGER_REFERENCE)")
 def test_from_reference_wraps_the_live_module_and_delegates_training(sd_diff):
     """B200GaussianDiffusion.from_reference(ref): denoiser weights, schedule buffers and spec_min/max are taken over from the live
     reference module (strict load), ``fs2`` is shared, and ``forward(infer=False)`` -- the training branch,

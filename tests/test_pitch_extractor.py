@@ -40,7 +40,7 @@ def test_oracle_vs_golden(pe_golden, i):
     assert 0.05 < float((g > 0).mean()) < 0.95                    # both voicing decisions occur
 
 
-@pytest.mark.skipif(not ref_shim.available(), reason="needs /root/reference (build container only)")
+@pytest.mark.skipif(not ref_shim.available(), reason="needs the original BiSinger source tree (set BISINGER_REFERENCE)")
 def test_oracle_vs_live_reference():
     from make_golden_pe import build_reference_pe
     ns = ref_shim.load()
