@@ -796,8 +796,7 @@ void HifiganPlan::enqueue(Workspace& w, const float* mel, const float* f0, const
                     } else if (j + 1 < nk) {
                         a.mode = j == 0 ? 1 : 2;
                     } else {
-                        a.mode = 3;
-                        if (nk == 1) { a.mode = 3; }
+                        a.mode = nk == 1 ? 4 : 3;   // a single ResBlock has no MRF sum to add to
                         a.out = last_stage ? static_cast<void*>(w.X0.p) : static_cast<void*>(w.upin[up_sel ^ 1].p);
                         a.out_bf16 = last_stage ? 0 : 1;
                         a.slope_out = last_stage ? 0.01f : kLrelu;

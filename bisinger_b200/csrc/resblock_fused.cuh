@@ -38,10 +38,11 @@ struct ResblockArgs {
     const float* bias1;
     const float* bias2;
     const __half* a_in;          // the tensor behind amap (residual rows)
-    void* out;                   // mode 0: next a = fp16 lrelu(y, 0.1); mode 3: fp16 or bf16 lrelu(sum, slope_out)
-    __half* sum;                 // modes 1-3: MRF accumulator (fp16, raw)
+    void* out;                   // mode 0: next a = fp16 lrelu(y, 0.1); modes 3-4: the fp16 or bf16 stage output (see mode)
+    __half* sum;                 // modes 1-3: MRF accumulator (fp16, raw); not touched in modes 0 and 4
     int mode;                    // 0: a_out = lrelu(y) | 1: sum = y c0 | 2: sum += y c0 | 3: out = lrelu(sum + y c0, slope_out)
-    int out_bf16;                // mode 3: out is bf16 (operand of the next stage's transposed convolution) instead of fp16
+                                 // | 4: out = lrelu(y c0, slope_out) (the only ResBlock of a single-kernel MRF: no sum to read)
+    int out_bf16;                // modes 3-4: out is bf16 (operand of the next stage's transposed convolution) instead of fp16
     float c0, slope_out;
     int w_slots;                 // weight tiles the shared-memory weight area holds
     int w_resident;              // 2: all weight tiles of both convolutions are loaded once per CTA (2 * n_wtiles <= w_slots); 1: conv1's tiles
@@ -443,7 +444,7 @@ __global__ void __launch_bounds__(kRbThreads, 1) resblock_iter_kernel(const __gr
                 if (ok) {
                     ldg256(xrow + c, xa);        // 16 fp16 each
                     ldg256(xrow + c + 16, xb);
-                    if (args.mode >= 2) {
+                    if (args.mode == 2 || args.mode == 3) {
                         ldg256(args.sum + row * C + c, sa);
                         ldg256(args.sum + row * C + c + 16, sb);
                     }
@@ -474,7 +475,7 @@ __global__ void __launch_bounds__(kRbThreads, 1) resblock_iter_kernel(const __gr
 #pragma unroll
                     for (int i = 0; i < 16; ++i) {
                         float s0 = y[2 * i] * args.c0, s1 = y[2 * i + 1] * args.c0;
-                        if (args.mode >= 2) {
+                        if (args.mode == 2 || args.mode == 3) {
                             const uint32_t ps = __float_as_uint(i < 8 ? sa[i] : sb[i - 8]);
                             const float2 s2 = __half22float2(*reinterpret_cast<const __half2*>(&ps));
                             s0 += s2.x; s1 += s2.y;

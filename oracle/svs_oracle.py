@@ -559,3 +559,36 @@ def snr_db(ref: Tensor, out: Tensor) -> float:
     num = (ref * ref).sum()
     den = ((ref - out) ** 2).sum().clamp_min(1e-300)
     return float(10.0 * torch.log10(num / den))
+
+
+def frame_snr_db(ref: Tensor, out: Tensor, hop: int = 128) -> float:
+    """Local counterpart of snr_db for one utterance: the mean signal power of the whole of ``ref`` over the error energy of
+    the worst ``hop``-sample frame, in dB (float64).  A defect confined to a few frames is diluted in the global SNR but not
+    here.  Frames are measured against the utterance's power, not their own: quiet and unvoiced frames would make a
+    per-frame ratio unstable.  A ragged last frame is averaged over the samples it has."""
+    ref = ref.double().flatten()
+    out = out.double().flatten()
+    assert ref.shape == out.shape and ref.numel() > 0
+    err = (ref - out) ** 2
+    n = err.numel() // hop * hop
+    frames = err[:n].reshape(-1, hop).mean(1)
+    if n < err.numel():
+        frames = torch.cat([frames, err[n:].mean()[None]])
+    return float(10.0 * torch.log10((ref * ref).mean() / frames.max().clamp_min(1e-300)))
+
+
+def wav_rows_db(ref: Tensor, out: Tensor, hop: int = 128) -> List[tuple]:
+    """(snr_db, frame_snr_db) of every batch row of a waveform [B, L] or [B, 1, L]: each row is its own utterance."""
+    assert ref.shape == out.shape
+    ref, out = ref.reshape(ref.shape[0], -1), out.reshape(out.shape[0], -1)
+    return [(snr_db(r, o), frame_snr_db(r, o, hop)) for r, o in zip(ref, out)]
+
+
+def assert_wav_rows(ref: Tensor, out: Tensor, snr_min_db: float, frame_min_db: float, hop: int = 128) -> None:
+    """Every batch row meets both bounds.  The figures of all rows are printed first (pytest -s shows them), so a failure
+    reports the rows that passed as well."""
+    rows = wav_rows_db(torch.as_tensor(ref), torch.as_tensor(out), hop)
+    print("wav rows (SNR dB, worst-frame dB):", ", ".join(f"({s:.1f}, {f:.1f})" for s, f in rows))
+    for b, (s, f) in enumerate(rows):
+        assert s >= snr_min_db and f >= frame_min_db, \
+            f"batch row {b}: SNR {s:.1f} dB (>= {snr_min_db}), worst frame {f:.1f} dB (>= {frame_min_db})"

@@ -193,7 +193,7 @@ def test_gpu_mel_to_wav_chain(dev):
         pytest.skip("a voicing logit within rounding of 0 flipped; the chain comparison needs identical decisions")
     from bisinger_b200 import mel_to_wav
     wav = mel_to_wav(mel.to(dev), gen, pe, rand_ini=vin["rand_ini"].to(dev), src_noise=vin["src_noise"].to(dev)).cpu()
-    assert O.snr_db(wref[:, 0], wav) >= 40.0
+    O.assert_wav_rows(wref[:, 0], wav, 40.0, 33.0)    # waveform SNR and worst-frame bound of tests/test_gpu_vocoder_frames.py, per row
     assert mel_to_wav(mel.to(dev), gen, pe, seed=3).shape == (B, T * 128)        # production path: device-drawn source noise
 
 
