@@ -59,6 +59,7 @@ EXPORTS = (
     "bsg_abi_version", "bsg_last_error", "bsg_kernel_launch_count",
     "bsg_diffusion_plan_create", "bsg_diffusion_plan_destroy", "bsg_diffusion_sample", "bsg_diffusion_sample_plms", "bsg_diffnet_forward",
     "bsg_diffusion_time_kernel",
+    "bsg_diffusion_q_sample", "bsg_diffusion_p_sample", "bsg_diffnet_forward_steps", "bsg_diffusion_plms_update",
     "bsg_hifigan_plan_create", "bsg_hifigan_plan_destroy", "bsg_hifigan_forward", "bsg_hifigan_source",
     "bsg_pe_plan_create", "bsg_pe_plan_destroy", "bsg_pe_forward",
     "bsg_fft_plan_create", "bsg_fft_plan_destroy", "bsg_fft_forward", "bsg_fft_forward_masked",
@@ -90,6 +91,11 @@ def lib() -> C.CDLL:
     L.bsg_diffusion_sample_plms.argtypes = [vp, fp, fp, fp, C.c_ulonglong, fp, C.POINTER(C.c_float), ip, ip, ip, fp, fp, vp]
     L.bsg_diffnet_forward.argtypes = [vp, fp, ip, fp, ip, ip, fp, vp]
     L.bsg_diffusion_time_kernel.argtypes = [vp, ip, ip, ip, ip, C.POINTER(C.c_float), vp]
+    tp, ull = C.POINTER(C.c_int), C.c_ulonglong
+    L.bsg_diffusion_q_sample.argtypes = [vp, fp, tp, fp, ull, ip, ip, fp, vp]
+    L.bsg_diffusion_p_sample.argtypes = [vp, fp, tp, fp, ull, fp, ull, ip, ip, ip, fp, vp]
+    L.bsg_diffnet_forward_steps.argtypes = [vp, fp, tp, fp, ull, ip, ip, fp, vp]
+    L.bsg_diffusion_plms_update.argtypes = [vp, fp, tp, C.POINTER(C.c_float), ip, ip, fp, fp, fp, fp, ip, ip, fp, vp]
     L.bsg_hifigan_plan_create.argtypes = [C.POINTER(HifiganConfig), C.POINTER(C.c_float), C.c_size_t, C.c_int, C.POINTER(vp)]
     L.bsg_hifigan_plan_destroy.argtypes = [vp]
     L.bsg_hifigan_plan_destroy.restype = None

@@ -86,6 +86,40 @@ int bsg_diffnet_forward(bsg_diffusion_plan* plan, const float* spec, int t, cons
     });
 }
 
+int bsg_diffusion_q_sample(bsg_diffusion_plan* plan, const float* x_start, const int* t, const float* noise, unsigned long long seed, int B,
+                           int T, float* x_out, void* stream) {
+    return guarded([&] {
+        B200_CHECK(plan, "null plan");
+        plan->impl.q_sample(x_start, t, noise, seed, B, T, x_out, static_cast<cudaStream_t>(stream));
+    });
+}
+
+int bsg_diffusion_p_sample(bsg_diffusion_plan* plan, const float* x, const int* t, const float* cond, unsigned long long cond_tag,
+                           const float* noise, unsigned long long seed, int clip_denoised, int B, int T, float* x_out, void* stream) {
+    return guarded([&] {
+        B200_CHECK(plan, "null plan");
+        plan->impl.p_sample(x, t, cond, cond_tag, noise, seed, clip_denoised != 0, B, T, x_out, static_cast<cudaStream_t>(stream));
+    });
+}
+
+int bsg_diffnet_forward_steps(bsg_diffusion_plan* plan, const float* spec, const int* t, const float* cond, unsigned long long cond_tag, int B,
+                              int T, float* eps_out, void* stream) {
+    return guarded([&] {
+        B200_CHECK(plan, "null plan");
+        plan->impl.denoise_steps(spec, t, cond, cond_tag, B, T, eps_out, static_cast<cudaStream_t>(stream));
+    });
+}
+
+int bsg_diffusion_plms_update(bsg_diffusion_plan* plan, const float* x, const int* t, const float* alphas_cumprod_host, int interval, int n_eps,
+                              const float* eps0, const float* eps1, const float* eps2, const float* eps3, int B, int T, float* x_out,
+                              void* stream) {
+    return guarded([&] {
+        B200_CHECK(plan, "null plan");
+        const float* eps[4] = {eps0, eps1, eps2, eps3};
+        plan->impl.plms_update(x, t, alphas_cumprod_host, interval, n_eps, eps, B, T, x_out, static_cast<cudaStream_t>(stream));
+    });
+}
+
 int bsg_diffusion_time_kernel(bsg_diffusion_plan* plan, int which, int B, int T, int reps, float* avg_ms, void* stream) {
     return guarded([&] {
         B200_CHECK(plan && avg_ms, "null argument");

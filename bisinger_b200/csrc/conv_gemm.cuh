@@ -68,7 +68,15 @@ enum : int {
     EPI_RELU_BF16 = 4,  // (acc+bias)*c0 [ReLU] -> hi/lo                         (net.py:126-128)
     EPI_POSTERIOR = 5,  // eps=acc+bias -> DDPM posterior update of x_t          (shallow_diffusion_tts.py:149-166)
     EPI_BIAS_ACT = 6,   // HiFi-GAN: y = acc+bias (+res) ; writes f32 and/or lrelu(y) bf16
+    // the same epilogues with a diffusion step per batch item (ConvGemmArgs::steps): a row tile never spans two batch items, so
+    // each tile looks up its item's step once.  Separate instantiations: the uniform-step kernels stay exactly as they are.
+    EPI_INPROJ_STEPS = 7,
+    EPI_RES_SKIP_STEPS = 8,
+    EPI_POSTERIOR_STEPS = 9,
 };
+__host__ __device__ constexpr int epi_base(int epi) {
+    return epi == EPI_INPROJ_STEPS ? EPI_INPROJ : (epi == EPI_RES_SKIP_STEPS ? EPI_RES_SKIP : (epi == EPI_POSTERIOR_STEPS ? EPI_POSTERIOR : epi));
+}
 
 struct EpiParams {
     const float* bias;         // [N_total]
@@ -95,6 +103,18 @@ struct EpiParams {
     uint8_t* out8;             // INPROJ: also write e4m3(x + d) [rows][out_pitch] (A operand of the fp8 correction MMAs), or null
 };
 
+// A diffusion step per batch item (the *_STEPS epilogues).  INPROJ / RES_SKIP: dvec points at the embedding of step 0 and
+// item b reads dvec + t_of_b[b] * dvec_stride.  POSTERIOR: c0..c4 of item b are coef[5b .. 5b+4] (c4 = 0 where t_b == 0), the
+// device noise of item b is Philox stream k_last - t_of_b[b] (the executed step at which the sampler reaches t_b), and
+// clip = 0 skips the clamp of x0 (clip_denoised=False).
+struct StepRows {
+    const int* t_of_b;     // device int32 [B]
+    const float* coef;     // device f32 [B][5]
+    int dvec_stride;
+    int k_last;
+    int clip;
+};
+
 struct ConvGemmArgs {
     CUtensorMap amap[4];   // A sources: (hi, lo) pairs, box = 64 channels x a_rows rows
     CUtensorMap wmap[2];   // packed weights hi / lo
@@ -112,6 +132,7 @@ struct ConvGemmArgs {
                            //    per weight tile that streaming the weights per tile left the kernel bound by TMA round trips
                            //    (~150 cycles per MMA whatever N: profiles/r01_i)
     unsigned long long* trace;   // optional [grid][16] cycle counters of the three roles (tests/tools/gpu_probe.py tracetarget), or null
+    StepRows steps;        // the *_STEPS epilogues only (kept behind every other member so that their offsets do not move)
 };
 
 // mbar_wait that adds the cycles spent waiting to *acc when tracing
@@ -295,7 +316,10 @@ enum : int {
 // FULL: all 32 rows of the warp are inside the batch (no row predicates).  Rows t >= L are never stored.
 template <int N_TILE, int EPI, bool FULL, bool OUT16>
 __device__ __forceinline__ void run_epilogue(const EpiParams& e, int Lrows, uint32_t tacc, int b, int t_warp, int n_tile, int grp,
-                                             float* stage, int lane) {
+                                             float* stage, int lane, const StepRows& sr) {
+    constexpr int BASE = epi_base(EPI);
+    constexpr bool kSteps = BASE != EPI;   // a diffusion step per batch item
+    (void)sr;
     const LanePos lp = lane_pos(lane);
     const float sc = e.acc_scale != 0.0f ? e.acc_scale : 1.0f;
     const long long row_w = static_cast<long long>(b) * Lrows + t_warp;   // global row of the warp's lane 0
@@ -322,13 +346,15 @@ __device__ __forceinline__ void run_epilogue(const EpiParams& e, int Lrows, uint
             for (int rp = 0; rp < 16; ++rp)
                 if (B200_ROW_OK(rp)) st2(p + rp * st, make_float2(o[rp].x + bias.x, o[rp].y + bias.y));
         }
-    } else if constexpr (EPI == EPI_INPROJ) {
+    } else if constexpr (BASE == EPI_INPROJ) {
+        const float* dv = e.dvec;
+        if constexpr (kSteps) dv += static_cast<long long>(__ldg(sr.t_of_b + b)) * sr.dvec_stride;
 #pragma unroll 1
         for (int c = c_begin; c < c_begin + kColsPerGrp; c += 32) {
             float2 o[16];
             ld_chunk_t(tacc, c, stage, lane, o, sc);
             const int n = n_tile * N_TILE + c + lp.cc;
-            const float2 bias = ldg2(e.bias + n), d = ldg2(e.dvec + n);
+            const float2 bias = ldg2(e.bias + n), d = ldg2(dv + n);
             const long long off0 = (row_w + lp.r0) * e.out_pitch + n, st = 2LL * e.out_pitch;
 #pragma unroll
             for (int rp = 0; rp < 16; ++rp) {
@@ -398,10 +424,14 @@ __device__ __forceinline__ void run_epilogue(const EpiParams& e, int Lrows, uint
                 }
             }
         }
-    } else if constexpr (EPI == EPI_RES_SKIP) {
+    } else if constexpr (BASE == EPI_RES_SKIP) {
         // residual half of the output projection: x <- (x + r + b) / sqrt(2)  (net.py:76-78); also writes the next
         // layer's conv input split(x + d_{l+1}) (net.py:69).  The skip half is not computed per layer: the skip sum is one
         // K = L*C GEMM over all gated activations at the end of the step (DiffusionPlan::enqueue_step).
+        [[maybe_unused]] const float* dv = nullptr;   // kSteps: d_{l+1} of this tile's batch item
+        if constexpr (kSteps) {
+            if (e.dvec != nullptr) dv = e.dvec + static_cast<long long>(__ldg(sr.t_of_b + b)) * sr.dvec_stride;
+        }
         const float rs2 = 0.70710678118654752440f;
         const long long st = 2LL * e.out_pitch;
         const int c0g = n_tile * N_TILE;
@@ -429,7 +459,11 @@ __device__ __forceinline__ void run_epilogue(const EpiParams& e, int Lrows, uint
             ld_chunk_t(tacc, c, stage, lane, o, sc);
             const float2 bias = ldg2(e.bias + cl);
             float2 d = make_float2(0.f, 0.f);
-            if (e.dvec != nullptr) d = ldg2(e.dvec + cl);
+            if constexpr (kSteps) {
+                if (e.dvec != nullptr) d = ldg2(dv + cl);
+            } else {
+                if (e.dvec != nullptr) d = ldg2(e.dvec + cl);
+            }
 #pragma unroll
             for (int rp = 0; rp < 16; ++rp) {
                 if (B200_ROW_OK(rp)) {
@@ -457,7 +491,7 @@ __device__ __forceinline__ void run_epilogue(const EpiParams& e, int Lrows, uint
                     st_operand2<2>(e, make_float2(fmaxf((o[rp].x + bias.x) * e.c0, lo_clamp), fmaxf((o[rp].y + bias.y) * e.c0, lo_clamp)),
                                 off0 + rp * st);
         }
-    } else if constexpr (EPI == EPI_POSTERIOR) {
+    } else if constexpr (BASE == EPI_POSTERIOR) {
         // row-per-thread ownership: row t_warp + lane.  x_t lives in the reference layout [B][M][T] (T contiguous): lanes hold
         // consecutive t, so the per-channel accesses below are coalesced.  The channels are processed in chunks of 16 with all
         // loads of a chunk issued before the first use (one exposed DRAM latency per chunk instead of one per channel:
@@ -469,9 +503,18 @@ __device__ __forceinline__ void run_epilogue(const EpiParams& e, int Lrows, uint
         const long long row = row_w + lane;
         const long long LL = Lrows;
         const bool eps_only = (e.flags & 1) != 0;     // bsg_diffnet_forward: write the denoiser output, reference layout
+        // kSteps: posterior coefficients and noise stream of this tile's batch item (the uniform-step kernel reads e.c0..c4, e.step)
+        [[maybe_unused]] float k0 = 0.f, k1 = 0.f, k2 = 0.f, k3 = 0.f, k4 = 0.f;
+        [[maybe_unused]] unsigned int k_step = 0;
+        if constexpr (kSteps) {
+            const float* cf = sr.coef + 5 * b;
+            k0 = __ldg(cf); k1 = __ldg(cf + 1); k2 = __ldg(cf + 2); k3 = __ldg(cf + 3); k4 = __ldg(cf + 4);
+            k_step = static_cast<unsigned int>(sr.k_last - __ldg(sr.t_of_b + b));
+        }
         float* xt = e.f32_a + (static_cast<long long>(b) * M) * LL + t;
         const float* nz = (!eps_only && e.aux0) ? e.aux0 + (static_cast<long long>(b) * M) * LL + t : nullptr;
-        const bool draw = !eps_only && nz == nullptr && e.c4 != 0.0f;   // the noise of the t == 0 step is multiplied by zero (:165)
+        // the noise of the t == 0 step is multiplied by zero (:165)
+        const bool draw = !eps_only && nz == nullptr && (kSteps ? k4 : e.c4) != 0.0f;
         const unsigned long long seed = draw ? __ldg(e.seed_ptr) : 0ull;
         const float mask = (e.f32_b != nullptr && row_ok && e.mel2ph != nullptr && !(e.mel2ph[row] > 0)) ? 0.0f : 1.0f;
 #pragma unroll 1
@@ -497,18 +540,30 @@ __device__ __forceinline__ void run_epilogue(const EpiParams& e, int Lrows, uint
                 for (int q = 0; q < 4; ++q) {
                     // one Philox4x32-10 call yields the four normals of channels c0+4q .. c0+4q+3 at this (b, t)
                     float4 z4 = make_float4(0.f, 0.f, 0.f, 0.f);
-                    if (draw) z4 = philox_normal4(seed, e.step, (static_cast<uint64_t>(b) * (M / 4) + (c0 >> 2) + q) * LL + t);
+                    if (draw) z4 = philox_normal4(seed, kSteps ? k_step : e.step, (static_cast<uint64_t>(b) * (M / 4) + (c0 >> 2) + q) * LL + t);
                     zv[4 * q] = z4.x; zv[4 * q + 1] = z4.y; zv[4 * q + 2] = z4.z; zv[4 * q + 3] = z4.w;
                 }
             }
+            if constexpr (kSteps) {
 #pragma unroll
-            for (int i = 0; i < 16; ++i) {
-                const float eps = acc[i] + __ldg(e.bias + c0 + i);
-                const float x = xv[i];
-                float x0 = e.c0 * x - e.c1 * eps;                       // predict_start_from_noise (:134-138)
-                x0 = fminf(fmaxf(x0, -1.0f), 1.0f);                      // clamp_ (:153-154)
-                const float mean = e.c2 * x0 + e.c3 * x;                 // q_posterior (:140-147)
-                xv[i] = mean + e.c4 * zv[i];                             // (:166), c4 = 0 at t == 0
+                for (int i = 0; i < 16; ++i) {
+                    const float eps = acc[i] + __ldg(e.bias + c0 + i);
+                    const float x = xv[i];
+                    float x0 = k0 * x - k1 * eps;
+                    if (sr.clip) x0 = fminf(fmaxf(x0, -1.0f), 1.0f);   // clip_denoised=False skips the clamp
+                    const float mean = k2 * x0 + k3 * x;
+                    xv[i] = mean + k4 * zv[i];
+                }
+            } else {
+#pragma unroll
+                for (int i = 0; i < 16; ++i) {
+                    const float eps = acc[i] + __ldg(e.bias + c0 + i);
+                    const float x = xv[i];
+                    float x0 = e.c0 * x - e.c1 * eps;                       // predict_start_from_noise (:134-138)
+                    x0 = fminf(fmaxf(x0, -1.0f), 1.0f);                      // clamp_ (:153-154)
+                    const float mean = e.c2 * x0 + e.c3 * x;                 // q_posterior (:140-147)
+                    xv[i] = mean + e.c4 * zv[i];                             // (:166), c4 = 0 at t == 0
+                }
             }
 #pragma unroll
             for (int i = 0; i < 16; ++i) xt[static_cast<long long>(c0 + i) * LL] = xv[i];
@@ -857,7 +912,7 @@ __global__ void __launch_bounds__(kGemmThreads, 1) conv_gemm_kernel(const __grid
     constexpr int kTileRows = PAIR ? 2 * kTileM : kTileM;
     // Narrow tiles (N_TILE = 32: the last HiFi-GAN stage) are bound by the epilogue's latency chain, not by its width: instead of
     // idling, the second group of four epilogue warps takes every other tile (accumulator buffer = tile parity = group).
-    constexpr bool kAltTiles = epi_col_split(N_TILE) == 1 && EPI != EPI_POSTERIOR;
+    constexpr bool kAltTiles = epi_col_split(N_TILE) == 1 && epi_base(EPI) != EPI_POSTERIOR;
 
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~static_cast<uintptr_t>(1023));
@@ -1105,15 +1160,15 @@ __global__ void __launch_bounds__(kGemmThreads, 1) conv_gemm_kernel(const __grid
             const uint32_t tacc = tmem_base + (static_cast<uint32_t>(quad * 32) << 16) + acc * N_TILE;
             float* stage = xpose + (warp - 2) * kStageFloatsPerWarp;
             const int grp = (warp - 2) >> 2;
-            if constexpr (EPI == EPI_RES_SKIP || EPI == EPI_BIAS_ACT || EPI == EPI_GATE) {
+            if constexpr (epi_base(EPI) == EPI_RES_SKIP || EPI == EPI_BIAS_ACT || EPI == EPI_GATE) {
                 const int nu = unit + (kAltTiles ? 2 : 1) * n_workers;   // this group's next tile
                 if (nu < n_units && B200_UNIT_TO_TILE(nu) < args.num_tiles)
-                    prefetch_rmw_tile<N_TILE, EPI>(args, B200_UNIT_TO_TILE(nu), kTileRows, rank * kTileM + quad * 32, grp, lane);
+                    prefetch_rmw_tile<N_TILE, epi_base(EPI)>(args, B200_UNIT_TO_TILE(nu), kTileRows, rank * kTileM + quad * 32, grp, lane);
             }
             // the fp16x2 per-layer GEMMs (gate, residual) feed fp16x2 consumers: fp16 operand output decided at compile time
             if (MC && b >= args.B) { /* the odd row tile of the last unit does not exist */ }
-            else if (args.L - t_warp >= 32) run_epilogue<N_TILE, EPI, true, TERMS == 2 || TERMS == 4>(args.epi, args.L, tacc, b, t_warp, n_tile, grp, stage, lane);
-            else run_epilogue<N_TILE, EPI, false, TERMS == 2 || TERMS == 4>(args.epi, args.L, tacc, b, t_warp, n_tile, grp, stage, lane);
+            else if (args.L - t_warp >= 32) run_epilogue<N_TILE, EPI, true, TERMS == 2 || TERMS == 4>(args.epi, args.L, tacc, b, t_warp, n_tile, grp, stage, lane, args.steps);
+            else run_epilogue<N_TILE, EPI, false, TERMS == 2 || TERMS == 4>(args.epi, args.L, tacc, b, t_warp, n_tile, grp, stage, lane, args.steps);
             tc_fence_before();
             __syncwarp();
             if (lane == 0) {

@@ -72,6 +72,8 @@ struct LayerArgs {
     int epoch;             // 1-based count of launches since the counters were zeroed: a row tile is complete at 16 * epoch
     int flags_ablate;      // timing ablations (bit 1: no fp8 MMAs, bit 2: no fp16 MMAs)
     unsigned long long* trace;
+    const int* t_of_b;     // diffnet_layer_kernel<MC, true>: device int32 [B] diffusion step of each batch item; lut_t is then the
+                           //    embedding table of ALL steps [k_step][total layers][C] (kept last: the members above do not move)
 };
 
 // op j of a CTA pair that owns cnt row tiles (3 * cnt ops): kind 0 = gate GEMM of channel half h, 1 = residual GEMM, of local row tile n
@@ -207,7 +209,10 @@ __device__ __forceinline__ void tma_store_3d(const void* desc, uint32_t smem_src
 // the other pair).  At ~1.3 MB of L2->SM traffic per row tile and CTA, more than half of it weights, the 2-CTA kernel runs
 // into the L2->SM throughput limit (profiles/r01_h); only 33 such clusters fit on a B200, but 128 row-tile pairs over 33
 // clusters are the same 4 rounds as 256 row tiles over 74 pairs.
-template <int MC>
+// STEPS = true: a diffusion step per batch item (args.t_of_b).  A row tile never spans two batch items (tiles_per_batch tiles per
+// item), so the residual epilogue of a tile reads d_l and d_{l+1} of its item's step from the embedding table through L1 instead
+// of the per-layer shared-memory staging.
+template <int MC, bool STEPS = false>
 __global__ void __launch_bounds__(kLayerThreads, 1) diffnet_layer_kernel(const __grid_constant__ LayerArgs args) {
     using S = LayerSmem;
     constexpr int C = 256;
@@ -519,8 +524,12 @@ __global__ void __launch_bounds__(kLayerThreads, 1) diffnet_layer_kernel(const _
               // fp16(x + d_l)), vec[256,512) = d_{l+1}.  All epilogue warps are past the previous layer's last use.
               asm volatile("bar.sync 1, 256;" ::: "memory");
               const int c = threadIdx.x - 64;
-              vec[c] = lpar.bias_r[c] - args.lut_t[static_cast<size_t>(l) * C + c];
-              vec[256 + c] = has_next ? args.lut_t[static_cast<size_t>(l + 1) * C + c] : 0.0f;
+              if constexpr (STEPS) {   // the step embeddings are per batch item: subtracted / added per op below
+                  vec[c] = lpar.bias_r[c];
+              } else {
+                  vec[c] = lpar.bias_r[c] - args.lut_t[static_cast<size_t>(l) * C + c];
+                  vec[256 + c] = has_next ? args.lut_t[static_cast<size_t>(l + 1) * C + c] : 0.0f;
+              }
               asm volatile("bar.sync 1, 256;" ::: "memory");
           }
           for (int j = 0; j < n_ops; ++j, ++jg) {
@@ -613,6 +622,11 @@ __global__ void __launch_bounds__(kLayerThreads, 1) diffnet_layer_kernel(const _
                 // The residual stream is carried only as the fp16 conv input: x = fp16(x + d_cur) - d_cur (tests/tools/precision_study.py
                 // "state fp16": 1.5-2.2e-3 vs 1.2-1.3e-3 max mel error).  No fp32 x is read or written: the epilogue streams the conv
                 // input once more (32-channel boxes) and stores only the next layer's fp16 / e4m3 conv input.
+                const float* d_cur = nullptr;   // STEPS: d_l of this tile's step (d_{l+1} follows at + C)
+                if constexpr (STEPS) {
+                    const int tb = b < args.B ? __ldg(args.t_of_b + b) : 0;
+                    d_cur = args.lut_t + (static_cast<size_t>(tb) * args.total_layers + l) * C;
+                }
                 auto res_chunk = [&](int c, const uint32_t (&v)[32]) {   // 32 channels
                     const int cl = grp * 128 + c * 32;
                     const int q = q_op + 2 * c + grp;
@@ -638,7 +652,14 @@ __global__ void __launch_bounds__(kLayerThreads, 1) diffnet_layer_kernel(const _
 #pragma unroll
                         for (int hh = 0; hh < 2; ++hh) {
                             const int c4 = cl + 8 * k + 4 * hh;
-                            const float4 bb = lds128(vec_s + c4 * 4), dd = lds128(vec_s + (256 + c4) * 4);
+                            float4 bb = lds128(vec_s + c4 * 4), dd;
+                            if constexpr (STEPS) {
+                                const float4 dl = __ldg(reinterpret_cast<const float4*>(d_cur + c4));
+                                bb = make_float4(bb.x - dl.x, bb.y - dl.y, bb.z - dl.z, bb.w - dl.w);
+                                dd = has_next ? __ldg(reinterpret_cast<const float4*>(d_cur + C + c4)) : make_float4(0.f, 0.f, 0.f, 0.f);
+                            } else {
+                                dd = lds128(vec_s + (256 + c4) * 4);
+                            }
                             const float y0 = (y[4 * hh] + fmaf(__uint_as_float(v[8 * k + 4 * hh]), rscale, bb.x)) * rs2 + dd.x;
                             const float y1 = (y[4 * hh + 1] + fmaf(__uint_as_float(v[8 * k + 4 * hh + 1]), rscale, bb.y)) * rs2 + dd.y;
                             const float y2 = (y[4 * hh + 2] + fmaf(__uint_as_float(v[8 * k + 4 * hh + 2]), rscale, bb.z)) * rs2 + dd.z;

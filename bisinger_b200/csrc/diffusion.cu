@@ -133,13 +133,22 @@ __global__ void init_x_kernel(int mode, const float* __restrict__ fs2_mel, const
 // in fp32 on the host, same operation order).  write_x = 0: predictor of the first iteration -- only the operand copy for the next
 // denoiser evaluation is written, x itself stays.  mel_out != null (last iteration): denorm_spec(x') * (mel2ph > 0) (:268-272).
 // One thread per (b, t); x, e* are [B][M][T].
+// ROWS = true (bsg_diffusion_plms_update, a step per batch item): item b uses da, cx, ce = coef_b[3b .. 3b+2] instead of the scalars, and
+// the operand copy is written only when xin_hi != null (the step call writes none: the next denoiser call imports x itself).
+template <bool ROWS>
 __global__ void plms_update_kernel(int mode, int write_x, float da, float cx, float ce, float* __restrict__ x, const float* __restrict__ e0,
                                    const float* __restrict__ e1, const float* __restrict__ e2, const float* __restrict__ e3, int B, int T, int M,
                                    __nv_bfloat16* __restrict__ xin_hi, __nv_bfloat16* __restrict__ xin_lo, float* __restrict__ mel_out,
-                                   const float* __restrict__ smin, const float* __restrict__ smax, const int64_t* __restrict__ mel2ph) {
+                                   const float* __restrict__ smin, const float* __restrict__ smax, const int64_t* __restrict__ mel2ph,
+                                   const float* __restrict__ coef_b) {
     const long long r = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
     if (r >= static_cast<long long>(B) * T) return;
     const int b = static_cast<int>(r / T), t = static_cast<int>(r % T);
+    if constexpr (ROWS) {
+        da = coef_b[3 * b];
+        cx = coef_b[3 * b + 1];
+        ce = coef_b[3 * b + 2];
+    }
     const float mask = (mel_out != nullptr && mel2ph != nullptr && !(mel2ph[r] > 0)) ? 0.0f : 1.0f;
     for (int c = 0; c < M; ++c) {
         const long long i = (static_cast<long long>(b) * M + c) * T + t;
@@ -153,12 +162,27 @@ __global__ void plms_update_kernel(int mode, int write_x, float da, float cx, fl
         const float xv = x[i];
         const float xn = xv + da * (cx * xv - ce * prime);
         if (write_x) x[i] = xn;
-        float hf; __nv_bfloat16 h, l;
-        split_bf16(xn, hf, h, l);
-        xin_hi[r * M + c] = h;
-        if (xin_lo) xin_lo[r * M + c] = l;
+        if (!ROWS || xin_hi != nullptr) {
+            float hf; __nv_bfloat16 h, l;
+            split_bf16(xn, hf, h, l);
+            xin_hi[r * M + c] = h;
+            if (xin_lo) xin_lo[r * M + c] = l;
+        }
         if (mel_out != nullptr) mel_out[r * M + c] = ((xn + 1.0f) / 2.0f * (smax[c] - smin[c]) + smin[c]) * mask;
     }
+}
+
+// q_sample (shallow_diffusion_tts.py:203-208) with a step per batch item: x = sa_b * x_start + sb_b * noise, coef = [B][2] (sa_b, sb_b) =
+// (sqrt_alphas_cumprod[t_b], sqrt_one_minus_alphas_cumprod[t_b]).  noise == null: drawn from the stream of the sampler's start noise
+// (init_x_kernel), so that q_sample(t = K-1) with seed s is the start sample(seed = s) uses.  One thread per element of [B][M][T].
+__global__ void q_sample_kernel(const float* __restrict__ x_start, const float* __restrict__ noise, const float* __restrict__ coef,
+                                const unsigned long long* __restrict__ seed_ptr, int B, int M, int T, float* __restrict__ x_out) {
+    const long long xi = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
+    if (xi >= static_cast<long long>(B) * M * T) return;
+    const int b = static_cast<int>(xi / (static_cast<long long>(M) * T));
+    const float sa = coef[2 * b], sb = coef[2 * b + 1];
+    const float z = noise ? noise[xi] : philox_normal(__ldg(seed_ptr), 0xFFFFFFFFu, static_cast<uint64_t>(xi));
+    x_out[xi] = sa * x_start[xi] + sb * z;
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -183,6 +207,8 @@ struct DiffusionPlan::Workspace {
     DevBuf plms_eps[4];              // PLMS: the last four noise predictions [B][M][T]
     DevBuf layer_tab;                // fused layer kernel: LayerParams[L] (weight / conditioner-projection tensor maps, scales) in device memory
     DevBuf layer_flags;              // ... and the row-tile completion counters of a multi-layer launch [L][row tiles]
+    DevBuf t_of_b, step_coef;        // step calls: int32 [B] diffusion step of each batch item; f32 [B][5] posterior coefficients
+    unsigned long long cond_tag = 0; // step calls: caller's tag of the cond whose projections cp holds (0: none / unknown)
     cudaGraphExec_t graph = nullptr;
     bool graph_has_mask = false;
     cudaGraphExec_t plms_graph = nullptr;   // the PLMS loop for (plms_interval, plms_has_mask, plms_ac)
@@ -698,10 +724,19 @@ void DiffusionPlan::reset_dataflow(Workspace& w, cudaStream_t st) {
 }
 
 void DiffusionPlan::enqueue_step(Workspace& w, int t, int k_exec, const float* noise_k, bool last, bool use_mask, int tail,
-                                 cudaStream_t st, float* eps_out, int epoch) {
+                                 cudaStream_t st, float* eps_out, int epoch, int rows) {
     const int M = cfg.in_dims, H = cfg.hidden_size, C = cfg.residual_channels, L = cfg.residual_layers;
     const int B = w.B, T = w.T;
-    const float* lut_t = lut.as<float>() + static_cast<size_t>(t) * L * C;
+    // rows & kRowsNet: the DiffNet kernels look up each batch item's step in w.t_of_b (lut_t is then the whole table);
+    // rows & kRowsPost: the posterior update takes each item's coefficients from w.step_coef
+    const bool rows_net = (rows & kRowsNet) != 0;
+    const float* lut_t = lut.as<float>() + (rows_net ? 0 : static_cast<size_t>(t) * L * C);
+    StepRows sr{};
+    sr.t_of_b = w.t_of_b.as<int>();
+    sr.coef = w.step_coef.as<float>();
+    sr.dvec_stride = L * C;
+    sr.k_last = cfg.k_step - 1;
+    sr.clip = (rows & kRowsNoClip) ? 0 : 1;
     auto nz = [&](const DevBuf& b) { return b.p ? b.as<__nv_bfloat16>() : nullptr; };
 
     {   // input projection + ReLU (net.py:116-118); writes x and (x + d_0)
@@ -717,7 +752,8 @@ void DiffusionPlan::enqueue_step(Workspace& w, int t, int k_exec, const float* n
         a.epi.dvec = lut_t;
         a.epi.out_pitch = C;
         a.epi.out8 = use_fused ? w.xa8.as<uint8_t>() : nullptr;
-        launch_conv_gemm(256, terms_side, EPI_INPROJ, a, st);
+        a.steps = sr;
+        launch_conv_gemm(256, terms_side, rows_net ? EPI_INPROJ_STEPS : EPI_INPROJ, a, st);
         ++launches, ++g_launch_count;
     }
     if (use_fused && fused_stack) {
@@ -727,18 +763,24 @@ void DiffusionPlan::enqueue_step(Workspace& w, int t, int k_exec, const float* n
             B200_CUDA(cudaMemsetAsync(w.layer_flags.p, 0, w.layer_flags.bytes, st));
             epoch = 1;
         }
-        launch_diffnet_layer(fused_args(w, 0, L, lut_t, epoch), st, fused_mc);
+        LayerArgs la = fused_args(w, 0, L, lut_t, epoch);
+        la.t_of_b = sr.t_of_b;
+        launch_diffnet_layer(la, st, fused_mc, rows_net);
         ++launches, ++g_launch_count;
     } else {
         for (int l = 0; l < L; ++l) {
             if (use_fused) {
-                launch_diffnet_layer(fused_args(w, l, 1, lut_t), st, fused_mc);
+                LayerArgs la = fused_args(w, l, 1, lut_t);
+                la.t_of_b = sr.t_of_b;
+                launch_diffnet_layer(la, st, fused_mc, rows_net);
                 ++launches, ++g_launch_count;
                 continue;
             }
             launch_conv_gemm(256, terms, EPI_GATE, gate_args(w, l), st, gate_mode);
             ++launches, ++g_launch_count;
-            launch_conv_gemm(kResTile, terms, EPI_RES_SKIP, resskip_args(w, l, lut_t), st);
+            ConvGemmArgs ra = resskip_args(w, l, lut_t);
+            ra.steps = sr;
+            launch_conv_gemm(kResTile, terms, rows_net ? EPI_RES_SKIP_STEPS : EPI_RES_SKIP, ra, st);
             ++launches, ++g_launch_count;
         }
     }
@@ -771,7 +813,8 @@ void DiffusionPlan::enqueue_step(Workspace& w, int t, int k_exec, const float* n
             a.epi.step = static_cast<unsigned>(k_exec);
         }
         a.epi.out_pitch = M;
-        launch_conv_gemm(80, terms_side, EPI_POSTERIOR, a, st);
+        a.steps = sr;
+        launch_conv_gemm(80, terms_side, (tail == 0 && (rows & kRowsPost)) ? EPI_POSTERIOR_STEPS : EPI_POSTERIOR, a, st);
         ++launches, ++g_launch_count;
     }
 }
@@ -794,6 +837,7 @@ void DiffusionPlan::sample(const float* cond, const float* fs2_mel, const float*
                                                                                     lo ? w.cond_lo.as<__nv_bfloat16>() : nullptr, n);
         ++launches, ++g_launch_count;
         precompute_cond(w, st);
+        w.cond_tag = 0;
         const int mode = fs2_mel ? 0 : 1;
         init_x_kernel<<<static_cast<unsigned>((rows + 127) / 128), 128, 0, st>>>(
             mode, fs2_mel, start_noise, d_spec_min.as<float>(), d_spec_max.as<float>(), sched[K - 1].sqrt_ac, sched[K - 1].sqrt_1mac,
@@ -847,6 +891,15 @@ void DiffusionPlan::sample(const float* cond, const float* fs2_mel, const float*
     if (x_final) B200_CUDA(cudaMemcpyAsync(x_final, w.xt.p, rows * M * 4, cudaMemcpyDeviceToDevice, st));
 }
 
+// get_x_pred coefficients in fp32, same operation order as the reference (:175-180): x' = x + da * (cx * x - ce * eps')
+static void plms_coef(const float* alphas_cumprod, int t, int interval, float& da, float& cx, float& ce) {
+    const float a_t = alphas_cumprod[t], a_prev = alphas_cumprod[t - interval > 0 ? t - interval : 0];
+    const float a_t_sq = std::sqrt(a_t), a_prev_sq = std::sqrt(a_prev);
+    da = a_prev - a_t;
+    cx = 1.0f / (a_t_sq * (a_t_sq + a_prev_sq));
+    ce = 1.0f / (a_t_sq * (std::sqrt((1.0f - a_prev) * a_t) + std::sqrt((1.0f - a_t) * a_prev)));
+}
+
 // PLMS / PNDM sampler: the infer branch with hparams['pndm_speedup'] = interval (shallow_diffusion_tts.py:168-201,258-264).
 // Deterministic after the start; K/interval iterations, one denoiser evaluation each plus one more in the first.
 void DiffusionPlan::sample_plms(const float* cond, const float* fs2_mel, const float* start_noise, unsigned long long seed,
@@ -869,6 +922,7 @@ void DiffusionPlan::sample_plms(const float* cond, const float* fs2_mel, const f
                                                                                     lo ? w.cond_lo.as<__nv_bfloat16>() : nullptr, n);
         ++launches, ++g_launch_count;
         precompute_cond(w, st);
+        w.cond_tag = 0;
         init_x_kernel<<<static_cast<unsigned>((rows + 127) / 128), 128, 0, st>>>(
             fs2_mel ? 0 : 1, fs2_mel, start_noise, d_spec_min.as<float>(), d_spec_max.as<float>(), sched[K - 1].sqrt_ac, sched[K - 1].sqrt_1mac,
             d_seed.as<unsigned long long>(), B, T, M, w.xt.as<float>(), w.xin_hi.as<__nv_bfloat16>(),
@@ -877,21 +931,13 @@ void DiffusionPlan::sample_plms(const float* cond, const float* fs2_mel, const f
         B200_CUDA(cudaGetLastError());
     }
     if (mel2ph) B200_CUDA(cudaMemcpyAsync(w.mel2ph.p, mel2ph, rows * 8, cudaMemcpyDeviceToDevice, st));
-    // get_x_pred coefficients in fp32, same operation order as the reference (:175-180)
-    auto coef = [&](int t, float& da, float& cx, float& ce) {
-        const float a_t = alphas_cumprod[t], a_prev = alphas_cumprod[t - interval > 0 ? t - interval : 0];
-        const float a_t_sq = std::sqrt(a_t), a_prev_sq = std::sqrt(a_prev);
-        da = a_prev - a_t;
-        cx = 1.0f / (a_t_sq * (a_t_sq + a_prev_sq));
-        ce = 1.0f / (a_t_sq * (std::sqrt((1.0f - a_prev) * a_t) + std::sqrt((1.0f - a_t) * a_prev)));
-    };
     auto update = [&](int mode, int write_x, int t, const float* e0, const float* e1, const float* e2, const float* e3, bool last) {
         float da, cx, ce;
-        coef(t, da, cx, ce);
-        plms_update_kernel<<<static_cast<unsigned>((rows + 127) / 128), 128, 0, st>>>(
+        plms_coef(alphas_cumprod, t, interval, da, cx, ce);
+        plms_update_kernel<false><<<static_cast<unsigned>((rows + 127) / 128), 128, 0, st>>>(
             mode, write_x, da, cx, ce, w.xt.as<float>(), e0, e1, e2, e3, B, T, M, w.xin_hi.as<__nv_bfloat16>(),
             lo ? w.xin_lo.as<__nv_bfloat16>() : nullptr, last ? w.mel.as<float>() : nullptr, d_spec_min.as<float>(), d_spec_max.as<float>(),
-            mel2ph ? w.mel2ph.as<int64_t>() : nullptr);
+            mel2ph ? w.mel2ph.as<int64_t>() : nullptr, nullptr);
         ++launches, ++g_launch_count;
         B200_CUDA(cudaGetLastError());
     };
@@ -983,9 +1029,159 @@ void DiffusionPlan::denoise(const float* spec, int t, const float* cond, int B, 
     launches += 2, g_launch_count += 2;
     B200_CUDA(cudaGetLastError());
     precompute_cond(w, st);
+    w.cond_tag = 0;
     reset_dataflow(w, st);
     enqueue_step(w, t, 0, nullptr, false, false, 1, st, nullptr, 1);
     B200_CUDA(cudaMemcpyAsync(eps_out, w.eps.p, rows * M * 4, cudaMemcpyDeviceToDevice, st));
+}
+
+// ---------------------------------------------------------------------------------------------
+// step calls: q_sample / p_sample / DiffNet.forward / the PLMS update with a diffusion step per batch item
+// ---------------------------------------------------------------------------------------------
+
+// Checks 0 <= t[b] < limit; returns whether all items share one step
+static bool check_steps(const int* t, int B, int limit) {
+    B200_CHECK(t != nullptr, "t is required");
+    bool uniform = true;
+    for (int b = 0; b < B; ++b) {
+        B200_CHECK(t[b] >= 0 && t[b] < limit, "diffusion step t[" + std::to_string(b) + "] = " + std::to_string(t[b]) +
+                                                  " outside [0, " + std::to_string(limit) + ")");
+        uniform = uniform && t[b] == t[0];
+    }
+    return uniform;
+}
+
+// t (host) -> w.t_of_b; coef (host, n_coef floats per item, or none) -> w.step_coef
+void DiffusionPlan::stage_steps(Workspace& w, const int* t, const float* coef, int n_coef, cudaStream_t st) {
+    const size_t B = static_cast<size_t>(w.B);
+    if (w.t_of_b.p == nullptr) {
+        w.t_of_b.alloc(B * sizeof(int));
+        w.step_coef.alloc(B * 5 * sizeof(float));
+    }
+    B200_CUDA(cudaMemcpyAsync(w.t_of_b.p, t, B * sizeof(int), cudaMemcpyHostToDevice, st));
+    if (coef) B200_CUDA(cudaMemcpyAsync(w.step_coef.p, coef, B * n_coef * sizeof(float), cudaMemcpyHostToDevice, st));
+}
+
+// Conditioner projections of all layers for `cond`, unless the workspace already holds those of the same nonzero tag
+void DiffusionPlan::prepare_cond(Workspace& w, const float* cond, unsigned long long tag, cudaStream_t st) {
+    if (tag != 0 && tag == w.cond_tag) return;
+    const bool lo = terms_side == 3;
+    const size_t n = static_cast<size_t>(w.B) * w.T * cfg.hidden_size;
+    split_kernel<<<static_cast<unsigned>((n / 4 + 255) / 256 + 1), 256, 0, st>>>(cond, w.cond_hi.as<__nv_bfloat16>(),
+                                                                                lo ? w.cond_lo.as<__nv_bfloat16>() : nullptr, n);
+    ++launches, ++g_launch_count;
+    B200_CUDA(cudaGetLastError());
+    precompute_cond(w, st);
+    w.cond_tag = tag;
+}
+
+// x [B][M][T] -> the sampler state w.xt and its operand copy w.xin
+void DiffusionPlan::import_x(Workspace& w, const float* x, cudaStream_t st) {
+    const size_t rows = static_cast<size_t>(w.B) * w.T;
+    const int M = cfg.in_dims;
+    if (x != w.xt.as<float>()) B200_CUDA(cudaMemcpyAsync(w.xt.p, x, rows * M * 4, cudaMemcpyDeviceToDevice, st));
+    init_x_kernel<<<static_cast<unsigned>((rows + 127) / 128), 128, 0, st>>>(2, nullptr, x, nullptr, nullptr, 0.f, 0.f, nullptr, w.B, w.T, M,
+                                                                             nullptr, w.xin_hi.as<__nv_bfloat16>(),
+                                                                             terms_side == 3 ? w.xin_lo.as<__nv_bfloat16>() : nullptr);
+    ++launches, ++g_launch_count;
+    B200_CUDA(cudaGetLastError());
+}
+
+// A small host table copied to the device for the kernels of ONE call on `st`.  Stream-ordered allocation: another call on another stream
+// gets its own copy, and the memory goes back to the pool when the call's work is done.
+struct StreamTable {
+    void* p = nullptr;
+    cudaStream_t st;
+    StreamTable(const std::vector<float>& host, cudaStream_t s) : st(s) {
+        B200_CUDA(cudaMallocAsync(&p, host.size() * sizeof(float), st));
+        B200_CUDA(cudaMemcpyAsync(p, host.data(), host.size() * sizeof(float), cudaMemcpyHostToDevice, st));
+    }
+    ~StreamTable() { if (p) cudaFreeAsync(p, st); }
+    const float* f() const { return static_cast<const float*>(p); }
+};
+
+void DiffusionPlan::q_sample(const float* x_start, const int* t, const float* noise, unsigned long long seed, int B, int T, float* x_out,
+                             cudaStream_t st) {
+    B200_CHECK(B > 0 && T > 0, "empty batch");
+    B200_CHECK(x_start != nullptr && x_out != nullptr, "x_start and x_out are required");
+    check_steps(t, B, cfg.timesteps);
+    B200_CUDA(cudaSetDevice(device));
+    std::vector<float> coef(static_cast<size_t>(B) * 2);
+    for (int b = 0; b < B; ++b) {
+        coef[2 * b] = sched[t[b]].sqrt_ac;
+        coef[2 * b + 1] = sched[t[b]].sqrt_1mac;
+    }
+    const StreamTable tab(coef, st);
+    if (noise == nullptr) B200_CUDA(cudaMemcpyAsync(d_seed.p, &seed, sizeof(seed), cudaMemcpyHostToDevice, st));
+    const long long n = static_cast<long long>(B) * cfg.in_dims * T;
+    q_sample_kernel<<<static_cast<unsigned>((n + 255) / 256), 256, 0, st>>>(x_start, noise, tab.f(), d_seed.as<unsigned long long>(), B,
+                                                                           cfg.in_dims, T, x_out);
+    ++launches, ++g_launch_count;
+    B200_CUDA(cudaGetLastError());
+}
+
+void DiffusionPlan::p_sample(const float* x, const int* t, const float* cond, unsigned long long cond_tag, const float* noise,
+                             unsigned long long seed, bool clip_denoised, int B, int T, float* x_out, cudaStream_t st) {
+    B200_CHECK(B > 0 && T > 0, "empty batch");
+    B200_CHECK(x != nullptr && cond != nullptr && x_out != nullptr, "x, cond and x_out are required");
+    const bool uniform = check_steps(t, B, cfg.k_step);
+    B200_CUDA(cudaSetDevice(device));
+    Workspace& w = workspace(B, T);
+    const int M = cfg.in_dims, K = cfg.k_step;
+    // the existing uniform-step kernels unless the items' steps differ (or the clamp is to be skipped: only the per-item posterior has the flag)
+    const int rows = (uniform ? 0 : kRowsNet) | ((uniform && clip_denoised) ? 0 : kRowsPost) | (clip_denoised ? 0 : kRowsNoClip);
+    std::vector<float> coef(static_cast<size_t>(B) * 5);
+    for (int b = 0; b < B; ++b) {
+        const StepCoef& sc = sched[t[b]];
+        const float c[5] = {sc.c0, sc.c1, sc.c2, sc.c3, sc.sigma};   // sigma = 0 at t == 0: no noise (nonzero_mask, :165)
+        std::copy(c, c + 5, &coef[5 * static_cast<size_t>(b)]);
+    }
+    stage_steps(w, t, coef.data(), 5, st);
+    if (noise == nullptr) B200_CUDA(cudaMemcpyAsync(d_seed.p, &seed, sizeof(seed), cudaMemcpyHostToDevice, st));
+    prepare_cond(w, cond, cond_tag, st);
+    import_x(w, x, st);
+    reset_dataflow(w, st);
+    // device noise of item b: the stream sample() uses at the executed step K-1-t_b
+    enqueue_step(w, t[0], K - 1 - t[0], noise, false, false, 0, st, nullptr, 1, rows);
+    B200_CUDA(cudaMemcpyAsync(x_out, w.xt.p, static_cast<size_t>(B) * T * M * 4, cudaMemcpyDeviceToDevice, st));
+}
+
+void DiffusionPlan::denoise_steps(const float* spec, const int* t, const float* cond, unsigned long long cond_tag, int B, int T, float* eps_out,
+                                  cudaStream_t st) {
+    B200_CHECK(B > 0 && T > 0, "empty batch");
+    B200_CHECK(spec != nullptr && cond != nullptr && eps_out != nullptr, "spec, cond and eps_out are required");
+    const bool uniform = check_steps(t, B, cfg.k_step);
+    B200_CUDA(cudaSetDevice(device));
+    Workspace& w = workspace(B, T);
+    stage_steps(w, t, nullptr, 0, st);
+    prepare_cond(w, cond, cond_tag, st);
+    import_x(w, spec, st);
+    reset_dataflow(w, st);
+    enqueue_step(w, t[0], 0, nullptr, false, false, 1, st, eps_out, 1, uniform ? 0 : kRowsNet);
+}
+
+void DiffusionPlan::plms_update(const float* x, const int* t, const float* alphas_cumprod, int interval, int n_eps, const float* const* eps,
+                                int B, int T, float* x_out, cudaStream_t st) {
+    B200_CHECK(B > 0 && T > 0, "empty batch");
+    B200_CHECK(x != nullptr && x_out != nullptr && alphas_cumprod != nullptr, "x, alphas_cumprod and x_out are required");
+    B200_CHECK(interval >= 1, "interval must be >= 1");
+    B200_CHECK(n_eps >= 0 && n_eps <= 4, "n_eps must be 0 (predictor), 1 (two evaluations) or 2..4 (history terms)");
+    const int n_needed = n_eps == 0 ? 1 : (n_eps == 1 ? 2 : n_eps);
+    for (int j = 0; j < n_needed; ++j) B200_CHECK(eps[j] != nullptr, "eps" + std::to_string(j) + " is required for n_eps = " + std::to_string(n_eps));
+    check_steps(t, B, cfg.timesteps);
+    B200_CUDA(cudaSetDevice(device));
+    const int M = cfg.in_dims;
+    const size_t rows = static_cast<size_t>(B) * T;
+    // get_x_pred coefficients in fp32, same operation order as the reference (:175-180) and sample_plms; a_prev at max(t_b - interval, 0).
+    // An element-wise update: no workspace, no operand copy (the next denoiser call imports x itself).
+    std::vector<float> coef(static_cast<size_t>(B) * 3);
+    for (int b = 0; b < B; ++b) plms_coef(alphas_cumprod, t[b], interval, coef[3 * b], coef[3 * b + 1], coef[3 * b + 2]);
+    const StreamTable tab(coef, st);
+    if (x_out != x) B200_CUDA(cudaMemcpyAsync(x_out, x, rows * M * 4, cudaMemcpyDeviceToDevice, st));
+    plms_update_kernel<true><<<static_cast<unsigned>((rows + 127) / 128), 128, 0, st>>>(
+        n_eps, 1, 0.f, 0.f, 0.f, x_out, eps[0], eps[1], eps[2], eps[3], B, T, M, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, tab.f());
+    ++launches, ++g_launch_count;
+    B200_CUDA(cudaGetLastError());
 }
 
 }  // namespace b200

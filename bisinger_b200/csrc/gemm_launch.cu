@@ -144,9 +144,9 @@ void launch_inst(const ConvGemmArgs& args, cudaStream_t stream) {
 
 // One fused DiffNet layer (diffnet_layer.cuh): persistent CTA pairs over the 256-row tiles, or (mc) clusters of two pairs
 // with multicast weight tiles (weight tensor maps must then have 64-row boxes).
-template <int MC>
+template <int MC, bool STEPS>
 static void launch_layer_inst(const LayerArgs& args, cudaStream_t stream) {
-    auto kern = diffnet_layer_kernel<MC>;
+    auto kern = diffnet_layer_kernel<MC, STEPS>;
     static std::once_flag once;
     static cudaError_t attr_err = cudaSuccess;
     std::call_once(once, [&] { attr_err = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, LayerSmem::kTotal); });
@@ -158,6 +158,7 @@ static void launch_layer_inst(const LayerArgs& args, cudaStream_t stream) {
     const int max_clusters = max_active_clusters(kern, kCtas, kLayerThreads, LayerSmem::kTotal);
     if (args.n_row_tiles <= 0) return;
     B200_CHECK(args.n_layers == 1 || args.flags != nullptr, "a multi-layer launch needs the row-tile completion counters");
+    B200_CHECK(!STEPS || args.t_of_b != nullptr, "the per-item step variant needs the step table");
     B200_CHECK(args.a_rows >= kTileM && args.a_rows * 128 <= LayerSmem::kASlotBytes && args.a_rows % 8 == 0, "A halo box does not fit the shared-memory slot");
     const int units = MC ? (args.n_row_tiles + 1) / 2 : args.n_row_tiles;
     cudaLaunchConfig_t cfg{};
@@ -217,9 +218,12 @@ static void launch_layer_inst(const LayerArgs& args, cudaStream_t stream) {
     B200_CUDA(cudaGetLastError());
     if (chain) B200_CUDA(cudaEventRecord(ev, stream));
 }
-void launch_diffnet_layer(const LayerArgs& args, cudaStream_t stream, bool mc) {
-    if (mc) launch_layer_inst<1>(args, stream);
-    else launch_layer_inst<0>(args, stream);
+void launch_diffnet_layer(const LayerArgs& args, cudaStream_t stream, bool mc, bool steps) {
+    if (steps) {
+        if (mc) launch_layer_inst<1, true>(args, stream);
+        else launch_layer_inst<0, true>(args, stream);
+    } else if (mc) launch_layer_inst<1, false>(args, stream);
+    else launch_layer_inst<0, false>(args, stream);
 }
 
 int conv_gemm_weight_slots(int n_tile, int terms) {
@@ -253,6 +257,10 @@ void launch_conv_gemm(int n_tile, int terms, int epi, const ConvGemmArgs& args, 
     B200_CASE(256, 1, EPI_RELU_BF16) B200_CASE(256, 3, EPI_RELU_BF16) B200_CASE(128, 1, EPI_RELU_BF16) B200_CASE(128, 3, EPI_RELU_BF16)
     B200_PAIR(256, 1, EPI_RELU_BF16) B200_PAIR(256, 3, EPI_RELU_BF16) B200_PAIR(128, 1, EPI_RELU_BF16) B200_PAIR(128, 3, EPI_RELU_BF16)
     B200_CASE(80, 1, EPI_POSTERIOR) B200_CASE(80, 3, EPI_POSTERIOR)
+    // DiffNet with a diffusion step per batch item (step calls whose items are at different steps)
+    B200_CASE(256, 1, EPI_INPROJ_STEPS) B200_CASE(256, 3, EPI_INPROJ_STEPS)
+    B200_CASE(128, 1, EPI_RES_SKIP_STEPS) B200_CASE(128, 2, EPI_RES_SKIP_STEPS) B200_CASE(128, 3, EPI_RES_SKIP_STEPS)
+    B200_CASE(80, 1, EPI_POSTERIOR_STEPS) B200_CASE(80, 3, EPI_POSTERIOR_STEPS)
     // two CTA pairs per cluster with multicast weights
     B200_MC(256, 1, EPI_F32) B200_MC(256, 2, EPI_F32) B200_MC(256, 3, EPI_F32) B200_MC(128, 2, EPI_F32)
     B200_MC(256, 2, EPI_GATE) B200_MC(256, 2, EPI_RELU_BF16) B200_MC(256, 3, EPI_RELU_BF16)

@@ -23,6 +23,14 @@ public:
     void sample_plms(const float* cond, const float* fs2_mel, const float* start_noise, unsigned long long seed, const int64_t* mel2ph,
                      const float* alphas_cumprod, int interval, int B, int T, float* mel_out, float* x_final, cudaStream_t st);
     void denoise(const float* spec, int t, const float* cond, int B, int T, float* eps_out, cudaStream_t st);
+    // step calls (include/bisinger_b200.h): t is a host int32 [B], one diffusion step per batch item
+    void q_sample(const float* x_start, const int* t, const float* noise, unsigned long long seed, int B, int T, float* x_out, cudaStream_t st);
+    void p_sample(const float* x, const int* t, const float* cond, unsigned long long cond_tag, const float* noise, unsigned long long seed,
+                  bool clip_denoised, int B, int T, float* x_out, cudaStream_t st);
+    void denoise_steps(const float* spec, const int* t, const float* cond, unsigned long long cond_tag, int B, int T, float* eps_out,
+                       cudaStream_t st);
+    void plms_update(const float* x, const int* t, const float* alphas_cumprod, int interval, int n_eps, const float* const* eps, int B, int T,
+                     float* x_out, cudaStream_t st);
     float time_kernel(int which, int B, int T, int reps, cudaStream_t st);
 
     bsg_diffnet_config cfg;
@@ -56,8 +64,14 @@ private:
     ConvGemmArgs skipsum_args(Workspace& w);
     struct LayerArgs fused_args(Workspace& w, int l0, int n, const float* lut_t, int epoch = 1);
     void reset_dataflow(Workspace& w, cudaStream_t st);
+    // rows: per-item step variants of enqueue_step (kRowsNet: the DiffNet kernels read w.t_of_b; kRowsPost: the posterior update reads
+    // w.step_coef [B][5]; kRowsNoClip: ... without the clamp of x0).  0: every item at step t, the kernels sample() runs.
+    static constexpr int kRowsNet = 1, kRowsPost = 2, kRowsNoClip = 4;
     void enqueue_step(Workspace& w, int t, int k_exec, const float* noise_k, bool last, bool use_mask, int tail, cudaStream_t st,
-                      float* eps_out = nullptr, int epoch = 1);
+                      float* eps_out = nullptr, int epoch = 1, int rows = 0);
+    void stage_steps(Workspace& w, const int* t, const float* coef, int n_coef, cudaStream_t st);
+    void prepare_cond(Workspace& w, const float* cond, unsigned long long tag, cudaStream_t st);
+    void import_x(Workspace& w, const float* x, cudaStream_t st);
 
     std::vector<Layer> layers;
     PackedW inproj, outproj, skipall;   // skipall: skip_projection x the skip halves of all output projections, [C][L*C]

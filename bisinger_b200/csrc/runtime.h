@@ -205,7 +205,7 @@ void launch_conv_gemm(int n_tile, int terms, int epi, const ConvGemmArgs& args, 
 
 // One fused DiffNet layer (diffnet_layer.cuh); args.n_row_tiles == 0 only sets the kernel attributes up
 struct LayerArgs;
-void launch_diffnet_layer(const LayerArgs& args, cudaStream_t stream, bool mc = false);
+void launch_diffnet_layer(const LayerArgs& args, cudaStream_t stream, bool mc = false, bool steps = false);   // steps: diffnet_layer_kernel<MC, true>
 
 // One fused HiFi-GAN ResBlock1 iteration (resblock_fused.cuh) for channels in {32, 64, 128}; args.num_tiles == 0 only sets the kernel
 // attributes up.  resblock_weight_slots: weight tiles (C rows x 64 K-columns) its shared-memory weight area holds.

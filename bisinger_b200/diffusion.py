@@ -13,6 +13,8 @@ from __future__ import annotations
 
 import ctypes as C
 import math
+import weakref
+from collections import OrderedDict, deque
 from typing import Optional
 
 import numpy as np
@@ -107,14 +109,15 @@ class B200DiffNet(nn.Module):
         return torch.cat([sd[n].detach().to("cpu", torch.float32).reshape(-1) for n in names]).contiguous()
 
     def forward(self, spec, diffusion_step, cond):
-        """spec [B,1,M,T], diffusion_step [B] (all equal, as the sampler passes it, shallow_diffusion_tts.py:267),
-        cond [B,H,T] -> [B,1,M,T]."""
+        """spec [B,1,M,T], diffusion_step [B] (one step per batch row, as in p_losses; the sampler passes equal steps,
+        shallow_diffusion_tts.py:267), cond [B,H,T] -> [B,1,M,T]."""
         if self._standalone_plan is None:
             self._standalone_plan = DiffusionPlan(self, precision=_lib.DEFAULT_PRECISION)
-        t = int(diffusion_step.reshape(-1)[0].item())
-        if not bool((diffusion_step == t).all()):
-            raise RuntimeError("B200DiffNet: all batch rows must share one diffusion step (as in p_sample)")
-        return self._standalone_plan.denoise(spec, t, cond.transpose(1, 2))
+        steps = diffusion_step.reshape(-1)
+        t = int(steps[0].item())
+        if bool((steps == t).all()):
+            return self._standalone_plan.denoise(spec, t, cond.transpose(1, 2))
+        return self._standalone_plan.denoise_steps(spec, steps, cond)
 
 
 FP16_SAFE_BOUND = 3.0e4   # fp16 holds +-65504: the residual stream's worst-case bound must stay below half of that
@@ -224,6 +227,8 @@ class DiffusionPlan:
         self.M = M
         self.H = denoise_fn.encoder_hidden
         self.precision = precision
+        self._cond_seen = OrderedDict()   # (B, T) -> (key, weak reference to the cond tensor, tag) of the last step call, LRU
+        self._next_tag = 0
 
     def __del__(self):
         h = getattr(self, "_h", None)
@@ -241,6 +246,110 @@ class DiffusionPlan:
         out = torch.empty_like(spec)
         _lib.check(_lib.lib().bsg_diffnet_forward(self._h, _lib.dev_ptr(spec), int(t), _lib.dev_ptr(cond), B, T, _lib.dev_ptr(out),
                                                   _lib.current_stream_ptr(self.device)))
+        return out
+
+    # ---- step calls (bsg_diffusion_q_sample / _p_sample / bsg_diffnet_forward_steps / bsg_diffusion_plms_update) ----------------
+    # t: [B] integer tensor (any device) or a Python int / sequence; cond_bHT: [B,H,T] as the reference passes it (a transposed view of
+    # decoder_inp) -- converted to the plan's [B,T,H] layout, which costs nothing for such a view.
+
+    def _steps(self, t, B: int):
+        steps = torch.as_tensor(t).reshape(-1)
+        if steps.dtype.is_floating_point or steps.dtype == torch.bool:
+            raise RuntimeError(f"t must hold integer diffusion steps, got {steps.dtype}")
+        if steps.numel() == 1 and B > 1:
+            steps = steps.expand(B)
+        if steps.numel() != B:
+            raise RuntimeError(f"t has {steps.numel()} steps for a batch of {B}")
+        return (C.c_int * B)(*[int(v) for v in steps.tolist()])
+
+    COND_SHAPES = 6   # shapes whose cond identity is remembered (the plan's cached workspaces, kMaxShapes in csrc/plans.h)
+
+    def _cond(self, cond_bHT, B: int, T: int):
+        """cond [B,H,T] -> (the [B,T,H] tensor the plan reads -- the caller holds it until the call is enqueued -- and the tag).  The plan reuses the conditioner projections of all residual layers while
+        the tag stays the same, so the tag of a shape is kept only while the call sees the SAME tensor object (held by a weak reference:
+        nothing is kept alive) with the same storage pointer, version counter (bumped by every in-place write through any view), shape
+        and strides.  Anything else gets a new tag from a counter that never repeats, so a tag that is no longer remembered here -- the
+        tensor was freed, another one took its place, or its shape fell out of the LRU -- can never match what a workspace stores."""
+        if tuple(cond_bHT.shape) != (B, self.H, T):
+            raise RuntimeError(f"cond must be [B={B},H={self.H},T={T}], got {tuple(cond_bHT.shape)}")
+        if cond_bHT.device != self.device or cond_bHT.dtype != torch.float32:
+            cond_bHT = cond_bHT.to(self.device, torch.float32)   # a fresh tensor on every call: its tag changes with it
+        key = (cond_bHT.data_ptr(), cond_bHT._version, tuple(cond_bHT.shape), tuple(cond_bHT.stride()))
+        seen = self._cond_seen.pop((B, T), None)
+        if seen is not None and seen[0] == key and seen[1]() is cond_bHT:
+            tag = seen[2]
+        else:
+            self._next_tag += 1
+            tag = self._next_tag
+        self._cond_seen[(B, T)] = (key, weakref.ref(cond_bHT), tag)
+        while len(self._cond_seen) > self.COND_SHAPES:
+            self._cond_seen.popitem(last=False)
+        return cond_bHT.transpose(1, 2).contiguous(), C.c_ulonglong(tag)
+
+    def _x(self, x, name="x", like=None):
+        """[B,1,M,T] float32 on the plan's device; like: a tensor whose shape it must have exactly (the kernels index noise and noise
+        predictions with x's [B][M][T] geometry)."""
+        x = x.to(self.device, torch.float32).contiguous()
+        if x.dim() != 4 or x.shape[1] != 1 or x.shape[2] != self.M:
+            raise RuntimeError(f"{name} must be [B,1,M={self.M},T], got {tuple(x.shape)}")
+        if like is not None and x.shape != like.shape:
+            raise RuntimeError(f"{name} has shape {tuple(x.shape)}, x has {tuple(like.shape)}")
+        return x
+
+    def q_sample(self, x_start, t, noise=None, seed: Optional[int] = None):
+        """q_sample (shallow_diffusion_tts.py:203-208) with a step per batch row: x_start, noise [B,1,M,T].  noise=None: drawn on the
+        device from the start-noise stream of ``sample`` (``q_sample(x, K-1, seed=s)`` is the start ``sample(seed=s)`` uses)."""
+        x_start = self._x(x_start, "x_start")
+        B, _, M, T = x_start.shape
+        steps = self._steps(t, B)
+        noise = None if noise is None else self._x(noise, "noise", like=x_start)
+        out = torch.empty_like(x_start)
+        _lib.check(_lib.lib().bsg_diffusion_q_sample(self._h, _lib.dev_ptr(x_start), steps, _lib.dev_ptr(noise),
+                                                     C.c_ulonglong(_lib.resolve_seed(seed)), B, T, _lib.dev_ptr(out),
+                                                     _lib.current_stream_ptr(self.device)))
+        return out
+
+    def p_sample(self, x, t, cond_bHT, clip_denoised: bool = True, noise=None, seed: Optional[int] = None):
+        """p_sample (shallow_diffusion_tts.py:149-166) with a step per batch row; rows with t == 0 get no noise.  noise=None: drawn on
+        the device from the stream ``sample`` uses at that step (a uniform-t call with seed s draws what ``sample(seed=s)`` does)."""
+        x = self._x(x)
+        B, _, M, T = x.shape
+        steps = self._steps(t, B)
+        cond, tag = self._cond(cond_bHT, B, T)
+        noise = None if noise is None else self._x(noise, "noise", like=x)
+        out = torch.empty_like(x)
+        _lib.check(_lib.lib().bsg_diffusion_p_sample(self._h, _lib.dev_ptr(x), steps, _lib.dev_ptr(cond), tag, _lib.dev_ptr(noise),
+                                                     C.c_ulonglong(_lib.resolve_seed(seed)), int(bool(clip_denoised)), B, T,
+                                                     _lib.dev_ptr(out), _lib.current_stream_ptr(self.device)))
+        return out
+
+    def denoise_steps(self, spec, t, cond_bHT):
+        """DiffNet.forward(spec, t, cond) with a step per batch row: spec [B,1,M,T], t [B], cond [B,H,T] -> eps [B,1,M,T]."""
+        spec = self._x(spec, "spec")
+        B, _, M, T = spec.shape
+        steps = self._steps(t, B)
+        cond, tag = self._cond(cond_bHT, B, T)
+        out = torch.empty_like(spec)
+        _lib.check(_lib.lib().bsg_diffnet_forward_steps(self._h, _lib.dev_ptr(spec), steps, _lib.dev_ptr(cond), tag, B, T, _lib.dev_ptr(out),
+                                                        _lib.current_stream_ptr(self.device)))
+        return out
+
+    def plms_update(self, x, t, interval: int, n_eps: int, eps):
+        """get_x_pred (shallow_diffusion_tts.py:174-183) on the PLMS combination selected by n_eps (0: predictor eps[0]; 1: mean of
+        eps[0], eps[1]; 2..4: Adams-Bashforth with eps[0] = current, eps[1..] = noise_list[-1], [-2], [-3])."""
+        if self._alphas_cumprod is None:
+            raise RuntimeError("plms_update needs the 'alphas_cumprod' schedule buffer (pass it in sched=)")
+        x = self._x(x)
+        B, _, M, T = x.shape
+        steps = self._steps(t, B)
+        needed = 1 if n_eps == 0 else (2 if n_eps == 1 else n_eps)
+        if not 0 <= n_eps <= 4 or len(eps) != needed:
+            raise RuntimeError(f"n_eps = {n_eps} takes {needed} noise predictions, got {len(eps)}")
+        e = [self._x(v, f"eps[{j}]", like=x) for j, v in enumerate(eps)] + [None] * (4 - len(eps))
+        out = torch.empty_like(x)
+        _lib.check(_lib.lib().bsg_diffusion_plms_update(self._h, _lib.dev_ptr(x), steps, _lib.fptr(self._alphas_cumprod), int(interval),
+                                                        int(n_eps), *[_lib.dev_ptr(v) for v in e], B, T, _lib.dev_ptr(out),
+                                                        _lib.current_stream_ptr(self.device)))
         return out
 
     def time_kernel(self, which: int, B: int, T: int, reps: int = 40) -> float:
@@ -369,6 +478,7 @@ class B200GaussianDiffusion(nn.Module):
         self.register_buffer("spec_max", torch.FloatTensor(spec_max)[None, None, :keep])
         self.precision = precision
         self._plan: Optional[DiffusionPlan] = None
+        self.noise_list = deque(maxlen=4)   # PLMS history of p_sample_plms (the reference creates it in forward, :259)
 
     @classmethod
     def from_reference(cls, ref: nn.Module, hparams: Optional[dict] = None, precision: str = _lib.DEFAULT_PRECISION):
@@ -464,3 +574,40 @@ class B200GaussianDiffusion(nn.Module):
 
     def out2mel(self, x):
         return x
+
+    # ---- step methods of the reference (shallow_diffusion_tts.py:149-208), for callers that drive their own loop.  t is a [B] long
+    # tensor with one diffusion step per batch row.  Extra keyword arguments noise= / seed= as on the other entry points.  The
+    # training-side helpers (predict_start_from_noise, q_posterior, p_mean_variance, p_losses) are not provided: training runs on the
+    # wrapped reference.
+
+    @torch.no_grad()
+    def q_sample(self, x_start, t, noise=None, seed=None):
+        """x_start, noise [B,1,M,T] (:203-208).  noise=None: drawn on the device; ``q_sample(x, K-1, seed=s)`` is the start of
+        ``sample(seed=s)``."""
+        return self.plan.q_sample(x_start, t, noise, seed)
+
+    @torch.no_grad()
+    def p_sample(self, x, t, cond, clip_denoised=True, repeat_noise=False, noise=None, seed=None):
+        """One ancestral step (:159-166): x [B,1,M,T], t [B], cond [B,H,T].  With noise=None the noise is drawn on the device from the
+        stream ``sample`` uses at that step, so the reference loop with seed s reproduces ``sample(seed=s)``."""
+        if repeat_noise:
+            raise NotImplementedError("B200GaussianDiffusion.p_sample: repeat_noise=True is not supported (no reference call site uses it)")
+        return self.plan.p_sample(x, t, cond, clip_denoised, noise, seed)
+
+    @torch.no_grad()
+    def p_sample_plms(self, x, t, interval, cond, clip_denoised=True, repeat_noise=False):
+        """One PLMS step (:168-201) with the history in ``self.noise_list`` (reset it to an empty ``deque(maxlen=4)`` before a loop, as
+        the reference's forward does at :259).  Deterministic; clip_denoised / repeat_noise are unused, as in the reference."""
+        plan = self.plan
+        noise_list = self.noise_list
+        noise_pred = plan.denoise_steps(x, t, cond)
+        if len(noise_list) == 0:
+            x_pred = plan.plms_update(x, t, interval, 0, [noise_pred])
+            t_prev = (torch.as_tensor(t).reshape(-1) - interval).clamp(min=0)
+            noise_pred_prev = plan.denoise_steps(x_pred, t_prev, cond)
+            x_prev = plan.plms_update(x, t, interval, 1, [noise_pred, noise_pred_prev])
+        else:
+            hist = [noise_list[-1 - j] for j in range(min(len(noise_list), 3))]
+            x_prev = plan.plms_update(x, t, interval, 1 + len(hist), [noise_pred] + hist)
+        noise_list.append(noise_pred)
+        return x_prev

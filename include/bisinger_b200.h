@@ -118,6 +118,46 @@ int bsg_diffusion_sample_plms(bsg_diffusion_plan* plan, const float* cond, const
 int bsg_diffnet_forward(bsg_diffusion_plan* plan, const float* spec, int t, const float* cond, int B, int T,
                         float* eps_out, void* stream);
 
+/* Step calls: the public step methods of GaussianDiffusion for callers that drive their own loop, with one diffusion step per
+ * batch item.  Common arguments:
+ *   t         HOST int32 [B]: the step of each batch item (the reference's [B] long tensor).  0 <= t[b] < k_step (q_sample and
+ *             plms_update: < timesteps); out-of-range steps are an error.  When all items share one step the kernels of
+ *             bsg_diffusion_sample run; otherwise their per-item variants (each 128-/256-row tile belongs to one item and looks its
+ *             step up once).
+ *   x, x_out  device f32 [B][1][M][T] (may be the same buffer); cond device f32 [B][T][H] as in bsg_diffusion_sample.
+ *   cond_tag  the conditioner projections of all residual layers (about a fifth of a step's FLOPs) are kept in the (B, T) workspace
+ *             with the caller's tag.  A nonzero tag equal to the stored one reuses them, so a caller passes the same nonzero tag for
+ *             as long as cond is unchanged and a new one when it changes.  0 always recomputes.  bsg_diffusion_sample,
+ *             bsg_diffusion_sample_plms, bsg_diffnet_forward and workspace eviction clear the stored tag.
+ *   noise     device f32 [B][1][M][T] or NULL: drawn on the device (Philox, keyed by `seed`) from the stream bsg_diffusion_sample uses
+ *             at the same point, so that a loop of step calls with seed s reproduces bsg_diffusion_sample(seed = s) exactly. */
+
+/* q_sample (shallow_diffusion_tts.py:203-208): x_out = sqrt_alphas_cumprod[t_b] x_start + sqrt_one_minus_alphas_cumprod[t_b] noise.
+ * Device noise: the start noise of bsg_diffusion_sample, i.e. q_sample(norm_spec(fs2_mel)^T, t = K-1, seed = s) is its start. */
+int bsg_diffusion_q_sample(bsg_diffusion_plan* plan, const float* x_start, const int* t, const float* noise, unsigned long long seed, int B,
+                           int T, float* x_out, void* stream);
+
+/* p_sample (:149-166): one ancestral step of every item from its own t_b: eps = DiffNet(x, t, cond), x0 = clamp(c0 x - c1 eps) (no clamp
+ * when clip_denoised == 0), x_out = c2 x0 + c3 x + sigma_t noise, with no noise where t_b == 0 (:165).  Device noise of item b: the
+ * stream bsg_diffusion_sample draws at its executed step K-1-t_b. */
+int bsg_diffusion_p_sample(bsg_diffusion_plan* plan, const float* x, const int* t, const float* cond, unsigned long long cond_tag,
+                           const float* noise, unsigned long long seed, int clip_denoised, int B, int T, float* x_out, void* stream);
+
+/* DiffNet.forward(spec, t, cond) (usr/diff/net.py:107-130) with a step per item; eps_out device f32 [B][1][M][T]. */
+int bsg_diffnet_forward_steps(bsg_diffusion_plan* plan, const float* spec, const int* t, const float* cond, unsigned long long cond_tag, int B,
+                              int T, float* eps_out, void* stream);
+
+/* get_x_pred of p_sample_plms (:174-183) on the Adams-Bashforth combination of noise predictions (:188-199), per item with
+ * a_prev = alphas_cumprod[max(t_b - interval, 0)]; coefficients in fp32 on the host as bsg_diffusion_sample_plms computes them.
+ *   n_eps = 0: predictor, eps0 = the current prediction (x_pred of the first iteration, :189)
+ *           1: (eps0 + eps1) / 2, eps1 = the prediction at x_pred (:190-191)
+ *           2: (3 eps0 - eps1) / 2;  3: (23 eps0 - 16 eps1 + 5 eps2) / 12;  4: (55 eps0 - 59 eps1 + 37 eps2 - 9 eps3) / 24,
+ *              eps1..3 = noise_list[-1], [-2], [-3] (:192-197)
+ *   eps0..eps3 device f32 [B][1][M][T] (unused ones may be NULL); alphas_cumprod_host: host f32 [timesteps]. */
+int bsg_diffusion_plms_update(bsg_diffusion_plan* plan, const float* x, const int* t, const float* alphas_cumprod_host, int interval, int n_eps,
+                              const float* eps0, const float* eps1, const float* eps2, const float* eps3, int B, int T, float* x_out,
+                              void* stream);
+
 /* Measurement hook for bench.py's roofline line: average duration (ms, CUDA events on `stream`) of `reps` back-to-back
  * launches of one hot kernel at batch shape (B, T), cycling through the residual layers.
  *   which = 0: dilated-conv + conditioner GEMM with the sigmoid*tanh gate epilogue (net.py:67-74)            [unfused path]
