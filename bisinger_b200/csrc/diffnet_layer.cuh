@@ -1,7 +1,8 @@
 // The DiffNet ResidualBlocks (usr/diff/net.py:58-78) as ONE persistent 2-CTA kernel: one launch runs a range of layers
 // (normally all 20 of a diffusion step), row tiles flowing from layer to layer as soon as their inputs are complete.
 //
-// Per 256-row tile n (128 rows per CTA of the pair) three GEMM "ops" run on one producer / MMA / epilogue pipeline:
+// Per pair tile n (256 rows: one 128-row slab per CTA of the pair, see "Slabs" below) three GEMM "ops" run on one producer /
+// MMA / epilogue pipeline:
 //     G(n,0)  G(n,1)   : acc[256 x 256] = conv_dilated(xa)[:, gate | filter rows of channel half h]            (K = 3 x 256)
 //                        epilogue: + conditioner projection, sigmoid * tanh -> z (fp16, the all-layer z matrix)
 //     R(n)             : acc[256 x 256] = z[rows, this layer's columns] * W_res^T                               (K = 256)
@@ -29,9 +30,15 @@
 // Warps: 0 = operand producer (TMA), 1 = MMA issuer (leader CTA), 2..9 = epilogue (TMEM lane quadrant = warp % 4, two
 // column groups), 10 = epilogue-operand producer (TMA loads of the cp / conv-input boxes).
 //
-// Layers: row tile m of layer l reads halo rows of tiles m-1, m, m+1 of layer l-1; completion counters in global memory
-// (wait_inputs below) order that, the conv input ping-pongs between two buffers, and the deal of row tiles to CTA pairs rotates
-// per layer so that the uneven split (256 tiles over 74 pairs) averages out.
+// Slabs: the rows of an item are cut into ceil(T / 128) slabs of 128 rows, numbered across the batch (g = b * slabs_per_item + s).
+// Pair tile u runs slabs 2u and 2u + 1, one per CTA: each CTA stages its own A rows with its own TMA loads, so the two halves
+// of an M = 256 MMA may belong to two items: an item's last pair tile leaves at most 127 rows idle, not 255 (T = 1875: 15 slabs
+// per item, 240 pair tiles at B = 32 instead of 256 item-aligned 256-row tiles).  Only the last pair tile of an odd slab count
+// has an empty half.  A CTA's 128 rows never span two items.
+//
+// Layers: slab g of layer l reads halo rows of slabs g-1, g, g+1 (of the same item) of layer l-1 (dilation <= 128); completion
+// counters in global memory (wait_inputs below) order that, the conv input ping-pongs between two buffers, and the deal of
+// pair tiles to CTA pairs rotates per layer so that the uneven split (240 pair tiles over 74 pairs) averages out.
 #pragma once
 #include "conv_gemm.cuh"
 
@@ -58,8 +65,8 @@ struct LayerArgs {
     int layer0, n_layers;  // layers [layer0, layer0 + n_layers) run in this launch; total_layers: the last one writes no conv input
     int total_layers;
     int B, T;
-    int tiles_per_batch;   // ceil(T / 256)
-    int n_row_tiles;       // B * tiles_per_batch
+    int slabs_per_item;    // ceil(T / 128): slab g = b * slabs_per_item + s holds rows [128 s, 128 s + 128) of item b
+    int n_slabs;           // B * slabs_per_item; pair tile u runs slabs 2u (leader CTA) and 2u + 1
     int a_rows;            // rows of the xa halo boxes (128 + 2 * max dilation, multiple of 8)
     int z_pitch;           // elements per row of the z matrix (layer l owns columns [l*C, (l+1)*C))
     __half* z_out;         // z matrix base
@@ -67,16 +74,16 @@ struct LayerArgs {
     __half* xa16_out[2];   // conv input buffers as plain pointers (layer l writes [(l + 1) & 1])
     uint8_t* xa8_out[2];
     const float* lut_t;    // [total layers][C] step embeddings d_l of this diffusion step
-    int* flags;            // n_layers > 1: [total layers][n_row_tiles] completion counters: every launch adds 16 (epilogue warps per row tile)
+    int* flags;            // n_layers > 1: [total layers][n_slabs] completion counters: every launch adds 8 (epilogue warps per CTA)
                            //    to each; they are zeroed ONCE per sampling call, not per launch
-    int epoch;             // 1-based count of launches since the counters were zeroed: a row tile is complete at 16 * epoch
+    int epoch;             // 1-based count of launches since the counters were zeroed: a slab is complete at 8 * epoch
     int flags_ablate;      // timing ablations (bit 1: no fp8 MMAs, bit 2: no fp16 MMAs)
     unsigned long long* trace;
     const int* t_of_b;     // diffnet_layer_kernel<MC, true>: device int32 [B] diffusion step of each batch item; lut_t is then the
                            //    embedding table of ALL steps [k_step][total layers][C] (kept last: the members above do not move)
 };
 
-// op j of a CTA pair that owns cnt row tiles (3 * cnt ops): kind 0 = gate GEMM of channel half h, 1 = residual GEMM, of local row tile n
+// op j of a CTA pair that owns cnt pair tiles (3 * cnt ops): kind 0 = gate GEMM of channel half h, 1 = residual GEMM, of local pair tile n
 struct LayerOp {
     int kind, n, h;
 };
@@ -204,21 +211,20 @@ __device__ __forceinline__ void tma_store_3d(const void* desc, uint32_t smem_src
                  : "memory");
 }
 
-// MC = 1: clusters of FOUR CTAs = two pairs working on two consecutive row tiles with the same weights; every weight tile is
+// MC = 1: clusters of FOUR CTAs = two pairs working on two consecutive pair tiles with the same weights; every weight tile is
 // read from L2 once per cluster (each CTA loads a quarter of the N rows and multicasts it to the CTA of the same rank in
-// the other pair).  At ~1.3 MB of L2->SM traffic per row tile and CTA, more than half of it weights, the 2-CTA kernel runs
-// into the L2->SM throughput limit (profiles/r01_h); only 33 such clusters fit on a B200, but 128 row-tile pairs over 33
-// clusters are the same 4 rounds as 256 row tiles over 74 pairs.
-// STEPS = true: a diffusion step per batch item (args.t_of_b).  A row tile never spans two batch items (tiles_per_batch tiles per
-// item), so the residual epilogue of a tile reads d_l and d_{l+1} of its item's step from the embedding table through L1 instead
-// of the per-layer shared-memory staging.
+// the other pair).  At ~1.3 MB of L2->SM traffic per pair tile and CTA, more than half of it weights, the 2-CTA kernel runs
+// into the L2->SM throughput limit (profiles/r01_h); only 33 such clusters fit on a B200, but 120 units over 33 clusters
+// are the same 4 rounds as 240 pair tiles over 74 pairs.
+// STEPS = true: a diffusion step per batch item (args.t_of_b).  A CTA's slab never spans two batch items, so the residual epilogue
+// of each CTA reads d_l and d_{l+1} of its slab's step from the embedding table through L1 instead of the per-layer shared-memory
+// staging (the two CTAs of a pair tile may be at different steps).
 template <int MC, bool STEPS = false>
 __global__ void __launch_bounds__(kLayerThreads, 1) diffnet_layer_kernel(const __grid_constant__ LayerArgs args) {
     using S = LayerSmem;
     constexpr int C = 256;
     constexpr uint32_t kIdesc16 = umma_idesc_f16(2 * kTileM, 256, /*fp16=*/true);
     constexpr uint32_t kIdesc8 = umma_idesc_f8(2 * kTileM, 256, /*A e4m3*/ 0, /*B e5m2*/ 1);
-    constexpr int kTileRows = 2 * kTileM;
 
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~static_cast<uintptr_t>(1023));
@@ -248,17 +254,26 @@ __global__ void __launch_bounds__(kLayerThreads, 1) diffnet_layer_kernel(const _
     constexpr int kPairs = MC ? 2 : 1;
     const int cluster_id = static_cast<int>(blockIdx.x) / kClusterCtas;
     const int n_clusters = static_cast<int>(gridDim.x) / kClusterCtas;
-    // local row tile n of this pair is global row tile kPairs * (cluster_id + n * n_clusters) + pidx; with MC the odd one of the
-    // last unit may not exist: its loads are zero-filled by the TMA unit (batch index out of range) and nothing is stored
-    const int n_units = (args.n_row_tiles + kPairs - 1) / kPairs;
-    const int n_workers = kPairs * n_clusters;       // row-tile stride
-    // The units are dealt round-robin to the clusters, so n_units % n_clusters of them own one unit more than the rest (256 row
-    // tiles over 74 pairs: 34 pairs with 4, 40 with 3).  In a multi-layer launch the deal rotates from layer to layer, so that
+    // local pair tile n of this pair is global pair tile kPairs * (cluster_id + n * n_clusters) + pidx.  A slab past the last one
+    // (odd slab count; with MC also a missing pair tile of the last unit) gets batch index B: its loads are zero-filled by the TMA
+    // unit and nothing is stored or counted
+    const int n_pair_tiles = (args.n_slabs + 1) / 2;
+    const int n_units = (n_pair_tiles + kPairs - 1) / kPairs;
+    const int n_workers = kPairs * n_clusters;       // pair-tile stride
+    // The units are dealt round-robin to the clusters, so n_units % n_clusters of them own one unit more than the rest (240 pair
+    // tiles over 74 pairs: 18 pairs with 4, 56 with 3).  In a multi-layer launch the deal rotates from layer to layer, so that
     // over the layers every cluster gets the same share instead of the same clusters finishing last in every layer.
     const int rot = args.n_layers > 1 ? n_units % n_clusters : 0;
     auto layer_cluster = [&](int l) { return (cluster_id + (l - args.layer0) * rot) % n_clusters; };
-    auto layer_cnt = [&](int l) { return (n_units - layer_cluster(l) + n_clusters - 1) / n_clusters; };       // row tiles of this pair in layer l
+    auto layer_cnt = [&](int l) { return (n_units - layer_cluster(l) + n_clusters - 1) / n_clusters; };       // pair tiles of this pair in layer l
     auto layer_worker = [&](int l) { return kPairs * layer_cluster(l) + pidx; };                              // ... the first of them
+    // this CTA's slab of pair tile m: its index g, batch item b (B if the slab does not exist) and first row t0 in the item
+    struct Slab { int g, b, t0; };
+    auto slab_of = [&](int m) {
+        const int g = 2 * m + rank;
+        if (g >= args.n_slabs) return Slab{g, args.B, 0};
+        return Slab{g, g / args.slabs_per_item, (g % args.slabs_per_item) * kTileM};
+    };
 
     if (threadIdx.x == 32) {
         for (int s = 0; s < S::kAStages; ++s) { mbar_init(&afull_bar[s], 1); mbar_init(&aempty_bar[s], 1); }
@@ -282,18 +297,18 @@ __global__ void __launch_bounds__(kLayerThreads, 1) diffnet_layer_kernel(const _
 
     const bool tr_on = args.trace != nullptr;
     const int layer_end = args.layer0 + args.n_layers;
-    // Several layers in one launch: row tile m of layer l reads conv-input rows that the row tiles m-1, m, m+1 (of the same
-    // batch item) of layer l-1 wrote IN THIS LAUNCH, possibly on other SMs.  Each of their 16 epilogue warps fences its
-    // stores and bumps flags[l-1][tile]; a TMA-issuing thread polls (acquire) and orders the generic-proxy writes before
-    // its async-proxy reads.  Pairs therefore run ahead into the next layer wherever their inputs are ready: the partial
-    // last round of a layer (256 row tiles over 74 pairs) overlaps the next layer instead of idling.
-    auto wait_inputs = [&](int l, int m, long long& acc_wait) {
-        if (args.flags == nullptr || l == args.layer0) return;
+    // Several layers in one launch: slab g of layer l reads conv-input rows that the slabs g-1, g, g+1 (of the same batch item)
+    // of layer l-1 wrote IN THIS LAUNCH, possibly on other SMs.  Each of the 8 epilogue warps of the CTA that ran a slab fences
+    // its stores and bumps flags[l-1][slab]; a TMA-issuing thread of the reading CTA polls (acquire) and orders the generic-proxy
+    // writes before its async-proxy reads.  Pairs therefore run ahead into the next layer wherever their inputs are ready: the
+    // partial last round of a layer (240 pair tiles over 74 pairs) overlaps the next layer instead of idling.
+    auto wait_inputs = [&](int l, const Slab& sl, long long& acc_wait) {
+        if (args.flags == nullptr || l == args.layer0 || sl.b >= args.B) return;
         const long long t0w = tr_on ? clock64() : 0;
-        const int ti = m % args.tiles_per_batch;
-        const int lo = ti > 0 ? m - 1 : m, hi = (ti + 1 < args.tiles_per_batch) ? m + 1 : m;
-        const int* f = args.flags + static_cast<size_t>(l - 1) * args.n_row_tiles;
-        const int done = 2 * kEpiWarps * args.epoch;   // counters run on from launch to launch (no memset node between the kernels of a step)
+        const int g = sl.g, s = sl.t0 / kTileM;
+        const int lo = s > 0 ? g - 1 : g, hi = (s + 1 < args.slabs_per_item) ? g + 1 : g;
+        const int* f = args.flags + static_cast<size_t>(l - 1) * args.n_slabs;
+        const int done = kEpiWarps * args.epoch;   // counters run on from launch to launch (no memset node between the kernels of a step)
         for (int mm = lo; mm <= hi; ++mm) {
             int v;
             unsigned spins = 0;
@@ -307,7 +322,7 @@ __global__ void __launch_bounds__(kLayerThreads, 1) diffnet_layer_kernel(const _
                     const long long now = clock64();
                     if (t_start == 0) t_start = now;
                     if (now - t_start > 8000000000LL) {
-                        printf("diffnet_layer_kernel: block %d waited > 4 s for row tile %d of layer %d\n", blockIdx.x, mm, l - 1);
+                        printf("diffnet_layer_kernel: block %d waited > 4 s for slab %d of layer %d\n", blockIdx.x, mm, l - 1);
                         __trap();
                     }
                 }
@@ -349,11 +364,10 @@ __global__ void __launch_bounds__(kLayerThreads, 1) diffnet_layer_kernel(const _
             const int worker = layer_worker(l), n_ops = 3 * cnt;
             for (int j = 0; j < n_ops; ++j) {
                 const LayerOp op = layer_op(j, cnt);
-                const int m = worker + op.n * n_workers;
-                const int b = m / args.tiles_per_batch;
-                const int t0 = (m % args.tiles_per_batch) * kTileRows + rank * kTileM;
+                const Slab sl = slab_of(worker + op.n * n_workers);
+                const int b = sl.b, t0 = sl.t0;
                 if (op.kind == 0) {
-                    if (op.h == 0) wait_inputs(l, m, w_dep);
+                    if (op.h == 0) wait_inputs(l, sl, w_dep);
                     const int wrow = op.h * 256 + rank * 128;
                     for (int k8 = 0; k8 < 2; ++k8) {
                         for (int kk = 0; kk < 2; ++kk) {
@@ -465,11 +479,10 @@ __global__ void __launch_bounds__(kLayerThreads, 1) diffnet_layer_kernel(const _
             const int cnt = layer_cnt(l), worker = layer_worker(l), n_ops = 3 * cnt;
             for (int j = 0; j < n_ops; ++j) {
                 const LayerOp op = layer_op(j, cnt);
-                const int m = worker + op.n * n_workers;
-                const int b = m / args.tiles_per_batch;
-                const int row = (m % args.tiles_per_batch) * kTileRows + rank * kTileM;
+                const Slab sl = slab_of(worker + op.n * n_workers);
+                const int b = sl.b, row = sl.t0;
                 const int nb = op.kind == 0 ? kGateBoxes : kResBoxes;
-                if (op.kind == 1) wait_inputs(l, m, w_dep);   // the boxes of a residual op are rows of this layer's conv input
+                if (op.kind == 1) wait_inputs(l, sl, w_dep);   // the boxes of a residual op are rows of this layer's conv input
                 for (int i = 0; i < nb; ++i, ++q) {
                     const int s = q % S::kEStages;
                     if (q >= S::kEStages) mbar_wait_tr(&edone_bar[s], ((q / S::kEStages) - 1) & 1, tr_on, w_e);   // previous occupant consumed by its four warps
@@ -535,9 +548,9 @@ __global__ void __launch_bounds__(kLayerThreads, 1) diffnet_layer_kernel(const _
           for (int j = 0; j < n_ops; ++j, ++jg) {
             const LayerOp op = layer_op(j, cnt);
             const int acc = jg & 1;
-            const int m = worker + op.n * n_workers;
-            const int b = m / args.tiles_per_batch;
-            const int t = (m % args.tiles_per_batch) * kTileRows + rank * kTileM + r_box;   // this thread's row in the batch item
+            const Slab sl = slab_of(worker + op.n * n_workers);
+            const int b = sl.b;
+            const int t = sl.t0 + r_box;   // this thread's row in the batch item
             const bool row_ok = t < args.T && b < args.B;
             const long long row = static_cast<long long>(b) * args.T + t;
             mbar_wait_tr(&tfull_bar[acc], (jg >> 1) & 1, tr, w_f);
@@ -699,15 +712,15 @@ __global__ void __launch_bounds__(kLayerThreads, 1) diffnet_layer_kernel(const _
             tc_fence_before();
             __syncwarp();
             if (lane == 0) mbar_arrive_remote_relaxed(tempty_remote0 + acc * 8);   // TMEM reads ordered by tcgen05.wait::ld + fence
-            if (op.kind == 1 && args.flags != nullptr && l + 1 < layer_end) {
+            if (op.kind == 1 && args.flags != nullptr && l + 1 < layer_end && b < args.B) {
                 // this warp's rows of the next layer's conv input are written: make them visible device-wide, then count the
-                // warp in (16 warps per row tile; readers: wait_inputs).  The readers are TMA loads (async proxy) issued by OTHER
+                // warp in (8 warps per slab; readers: wait_inputs).  The readers are TMA loads (async proxy) issued by OTHER
                 // CTAs: the generic-proxy stores are ordered against the async proxy HERE, by the threads that made them (as
                 // publish_z does for the z rows), not only by the reader's fence after its acquire
                 asm volatile("fence.proxy.async.global;" ::: "memory");
                 __threadfence();
                 __syncwarp();
-                if (lane == 0) asm volatile("red.release.gpu.global.add.s32 [%0], 1;" ::"l"(args.flags + static_cast<size_t>(l) * args.n_row_tiles + m) : "memory");
+                if (lane == 0) asm volatile("red.release.gpu.global.add.s32 [%0], 1;" ::"l"(args.flags + static_cast<size_t>(l) * args.n_slabs + sl.g) : "memory");
             }
             if (tr) { if (op.kind == 0) t_gate += clock64() - t_op; else t_res += clock64() - t_op; }
           }

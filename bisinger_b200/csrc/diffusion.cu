@@ -206,7 +206,7 @@ struct DiffusionPlan::Workspace {
     CUtensorMap m_z8;
     DevBuf plms_eps[4];              // PLMS: the last four noise predictions [B][M][T]
     DevBuf layer_tab;                // fused layer kernel: LayerParams[L] (weight / conditioner-projection tensor maps, scales) in device memory
-    DevBuf layer_flags;              // ... and the row-tile completion counters of a multi-layer launch [L][row tiles]
+    DevBuf layer_flags;              // ... and the slab completion counters of a multi-layer launch [L][B * ceil(T / 128)]
     DevBuf t_of_b, step_coef;        // step calls: int32 [B] diffusion step of each batch item; f32 [B][5] posterior coefficients
     unsigned long long cond_tag = 0; // step calls: caller's tag of the cond whose projections cp holds (0: none / unknown)
     cudaGraphExec_t graph = nullptr;
@@ -243,6 +243,8 @@ DiffusionPlan::DiffusionPlan(const bsg_diffnet_config& c, const float* w, size_t
     B200_CHECK(M == 80, "this build is specialised for 80 mel bins");
     B200_CHECK(L >= 1 && c.k_step >= 1 && c.k_step <= c.timesteps, "bad layer/step counts");
     B200_CHECK(c.dilation_cycle >= 1 && (1 << (c.dilation_cycle - 1)) * 2 + kTileM <= kXaBoxRows, "dilation cycle too long for the halo tile");
+    // the fused layer kernel's slab dataflow waits only for the neighbouring 128-row slabs: the halo must not reach further
+    B200_CHECK((1 << (c.dilation_cycle - 1)) <= kTileM, "dilation longer than a slab");
     B200_CHECK(c.precision == BSG_PRECISION_BF16 || c.precision == BSG_PRECISION_BF16X3 || c.precision == BSG_PRECISION_FP16X2,
                "bad precision");
     // terms: the per-layer GEMMs (gate, residual, skip sum); terms_side: the once-per-step / once-per-batch GEMMs
@@ -507,8 +509,8 @@ DiffusionPlan::Workspace& DiffusionPlan::workspace(int B, int T) {
         }
         w->layer_tab.alloc(tab.size() * sizeof(LayerParams));
         B200_CUDA(cudaMemcpy(w->layer_tab.p, tab.data(), tab.size() * sizeof(LayerParams), cudaMemcpyHostToDevice));
-        const int n_row_tiles = B * ((T + 2 * kTileM - 1) / (2 * kTileM));
-        w->layer_flags.alloc(static_cast<size_t>(cfg.residual_layers) * n_row_tiles * sizeof(int));
+        const int n_slabs = B * ((T + kTileM - 1) / kTileM);
+        w->layer_flags.alloc(static_cast<size_t>(cfg.residual_layers) * n_slabs * sizeof(int));
     }
     w->bytes = pooled_bytes;
     {   // what the pool keeps beyond the live workspaces counts against the same budget
@@ -586,8 +588,8 @@ ConvGemmArgs DiffusionPlan::resskip_args(Workspace& w, int l, const float* lut_t
     return a;
 }
 
-// ResidualBlocks [l0, l0 + n) in one launch of the fused layer kernel (diffnet_layer.cuh): per 256-row tile the gate GEMM of both
-// channel halves + the residual GEMM; n > 1: row-tile dataflow across the layers (zero w.layer_flags before the launch)
+// ResidualBlocks [l0, l0 + n) in one launch of the fused layer kernel (diffnet_layer.cuh): per pair tile (two 128-row slabs) the
+// gate GEMM of both channel halves + the residual GEMM; n > 1: slab dataflow across the layers (zero w.layer_flags before the launch)
 LayerArgs DiffusionPlan::fused_args(Workspace& w, int l0, int n, const float* lut_t, int epoch) {
     const int C = cfg.residual_channels, L = cfg.residual_layers;
     LayerArgs a{};
@@ -601,8 +603,8 @@ LayerArgs DiffusionPlan::fused_args(Workspace& w, int l0, int n, const float* lu
     a.total_layers = L;
     a.B = w.B;
     a.T = w.T;
-    a.tiles_per_batch = (w.T + 2 * kTileM - 1) / (2 * kTileM);
-    a.n_row_tiles = a.B * a.tiles_per_batch;
+    a.slabs_per_item = (w.T + kTileM - 1) / kTileM;
+    a.n_slabs = a.B * a.slabs_per_item;
     a.a_rows = kXaBoxRows;
     a.z_pitch = L * C;
     a.z_out = w.z_hi.as<__half>();

@@ -142,7 +142,7 @@ void launch_inst(const ConvGemmArgs& args, cudaStream_t stream) {
 
 }  // namespace
 
-// One fused DiffNet layer (diffnet_layer.cuh): persistent CTA pairs over the 256-row tiles, or (mc) clusters of two pairs
+// One fused DiffNet layer (diffnet_layer.cuh): persistent CTA pairs over the pair tiles (two 128-row slabs), or (mc) clusters of two pairs
 // with multicast weight tiles (weight tensor maps must then have 64-row boxes).
 template <int MC, bool STEPS>
 static void launch_layer_inst(const LayerArgs& args, cudaStream_t stream) {
@@ -156,11 +156,13 @@ static void launch_layer_inst(const LayerArgs& args, cudaStream_t stream) {
     // the grid must be resident.  The grid is therefore sized from what the driver says fits on THIS context's share of the device
     // (see the co-residency notes at the launch below).
     const int max_clusters = max_active_clusters(kern, kCtas, kLayerThreads, LayerSmem::kTotal);
-    if (args.n_row_tiles <= 0) return;
-    B200_CHECK(args.n_layers == 1 || args.flags != nullptr, "a multi-layer launch needs the row-tile completion counters");
+    if (args.n_slabs <= 0) return;
+    B200_CHECK(args.n_layers == 1 || args.flags != nullptr, "a multi-layer launch needs the slab completion counters");
     B200_CHECK(!STEPS || args.t_of_b != nullptr, "the per-item step variant needs the step table");
     B200_CHECK(args.a_rows >= kTileM && args.a_rows * 128 <= LayerSmem::kASlotBytes && args.a_rows % 8 == 0, "A halo box does not fit the shared-memory slot");
-    const int units = MC ? (args.n_row_tiles + 1) / 2 : args.n_row_tiles;
+    B200_CHECK(args.n_slabs == args.B * args.slabs_per_item && args.slabs_per_item * kTileM >= args.T, "slab count does not match the shape");
+    const int pair_tiles = (args.n_slabs + 1) / 2;   // slabs 2u and 2u + 1
+    const int units = MC ? (pair_tiles + 1) / 2 : pair_tiles;
     cudaLaunchConfig_t cfg{};
     cfg.gridDim = dim3(kCtas * (units < max_clusters ? units : max_clusters));
     cfg.blockDim = dim3(kLayerThreads);

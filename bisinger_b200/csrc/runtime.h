@@ -203,7 +203,7 @@ int conv_gemm_weight_slots(int n_tile, int terms);
 // pair = 2: clusters of two such pairs with multicast weight tiles; weight tensor map box = n_tile/4 rows
 void launch_conv_gemm(int n_tile, int terms, int epi, const ConvGemmArgs& args, cudaStream_t stream, int pair = 0);
 
-// One fused DiffNet layer (diffnet_layer.cuh); args.n_row_tiles == 0 only sets the kernel attributes up
+// One fused DiffNet layer (diffnet_layer.cuh); args.n_slabs == 0 only sets the kernel attributes up
 struct LayerArgs;
 void launch_diffnet_layer(const LayerArgs& args, cudaStream_t stream, bool mc = false, bool steps = false);   // steps: diffnet_layer_kernel<MC, true>
 

@@ -122,8 +122,8 @@ int bsg_diffnet_forward(bsg_diffusion_plan* plan, const float* spec, int t, cons
  * batch item.  Common arguments:
  *   t         HOST int32 [B]: the step of each batch item (the reference's [B] long tensor).  0 <= t[b] < k_step (q_sample and
  *             plms_update: < timesteps); out-of-range steps are an error.  When all items share one step the kernels of
- *             bsg_diffusion_sample run; otherwise their per-item variants (each 128-/256-row tile belongs to one item and looks its
- *             step up once).
+ *             bsg_diffusion_sample run; otherwise their per-item variants (the 128 rows of each CTA belong to one item, whose
+ *             step it looks up once).
  *   x, x_out  device f32 [B][1][M][T] (may be the same buffer); cond device f32 [B][T][H] as in bsg_diffusion_sample.
  *   cond_tag  the conditioner projections of all residual layers (about a fifth of a step's FLOPs) are kept in the (B, T) workspace
  *             with the caller's tag.  A nonzero tag equal to the stored one reuses them, so a caller passes the same nonzero tag for
